@@ -8,7 +8,11 @@ Philox collision noise).  value = envs x ants x steps / time, whole job over all
 shard is fixed; N = 8 of the default workload is BASELINE.json configs[3]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4|cfg3|cfg2] [--envs E] [--evap lazy|tiles|dense]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...      # the UNMODIFIED reference (oracle/_ref) on the host cores
+
+--dump-outputs DIR writes the outputs of the last timed step (obs, agent_state, reward) as DIR/<name>.npy; the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 
 The timed region is ONE C call (ants_rollout over a device-resident action tape): per step one launch of the perception
 kernel and one of the block-per-environment kernel (update_k ; move of step_{k+1}); no Python between the steps.
@@ -260,7 +264,62 @@ def load_peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+# ----------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_BYTES = 64 * 10 ** 6          # at most this much array data in DIR
+
+
+def sample_outputs(obs, agent_state, reward):
+    """The outputs of one step as a caller of ants_rollout receives them -- obs (E,N,S,S,C) f32, agent_state (E,N,2)
+    f32, reward (E,N) f64 -- copied to the host with the env and ant axes flattened (row = env * N + ant).  When all
+    ants do not fit in DUMP_BYTES, the rows are a fixed sample: np.sort(RandomState(0).choice(E * N, n, replace=False)),
+    the same rows in every array."""
+    import torch
+    obs, agent_state, reward = (t.reshape(t.shape[0] * t.shape[1], *t.shape[2:]) for t in (obs, agent_state, reward))
+    n_all = obs.shape[0]
+    per_ant = obs[0].numel() * obs.element_size() + agent_state[0].numel() * agent_state.element_size() + reward.element_size()
+    n = min(n_all, (DUMP_BYTES - 3 * 4096) // per_ant)          # 4096: room for each .npy header
+    if n < n_all:
+        rows = torch.from_numpy(np.sort(np.random.RandomState(0).choice(n_all, n, replace=False))).to(obs.device)
+        obs, agent_state, reward = (t.index_select(0, rows) for t in (obs, agent_state, reward))
+    return {"obs": obs.cpu().numpy(), "agent_state": agent_state.cpu().numpy(), "reward": reward.cpu().numpy()}
+
+
+def write_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------- main arms
+def make_batch(args, rank=0, device=0):
+    """The inputs of one rank, ready for the first step: its envs from the drop-in generator, pheromones activated, the
+    first observation taken, and the action tapes (T, E, N) on the device.
+    -> (gen, batch, cell record format, rot_tape, ph_tape)."""
+    import torch
+    from antsrl_b200 import BatchedAnts
+    from antsrl_b200.generator import stack_states
+    wl = WORKLOADS[args.workload]
+    E = args.envs or wl["envs_per_gpu"]
+    N = wl["n_ants"]
+    K = args.steps
+    total_steps = max(args.warmup + 3 * K, args.late_start + K) + 2 * args.e2e_steps + 16
+    gen = make_generator(wl, total_steps + 10)
+    states = generate_states_parallel(wl, total_steps + 10, rank * E, E)
+    record = args.record if args.evap == "lazy" else "f64"
+    batch = BatchedAnts(gen.cfg, E, device=device, evap_mode=args.evap, rng_seed=20261018, env_id_base=rank * E,
+                        record=record)
+    batch.import_state(stack_states(states, gen.cfg["reward_kind"]))
+    del states
+    batch.activate_all_pheromones(np.ones((E, N, wl["n_phero"])) * 10.0)      # agent.initialize, collect_agent.py:100
+    rs = np.random.RandomState(12345 + rank)
+    n_tape = max(K, 32)                                                       # the pre-recorded action sequence
+    rot_tape = torch.from_numpy((rs.randint(0, 3, size=(n_tape, E, N)) - 1).astype(np.int8)).cuda()
+    ph_tape = torch.from_numpy(rs.randint(0, 3, size=(n_tape, E, N)).astype(np.int8)).cuda()
+    batch.observe()                                                           # main.py:88
+    return gen, batch, record, rot_tape, ph_tape
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -276,27 +335,14 @@ def run_ours(args):
     N = wl["n_ants"]
     K, W_ = args.steps, args.warmup
     late_start = args.late_start
-    total_steps = max(W_ + 3 * K, late_start + K) + 2 * args.e2e_steps + 16
 
     t_setup = time.perf_counter()
-    gen = make_generator(wl, total_steps + 10)
-    states = generate_states_parallel(wl, total_steps + 10, rank * E, E)
-    from antsrl_b200 import BatchedAnts
-    from antsrl_b200.generator import stack_states
-    record = args.record if args.evap == "lazy" else "f64"
-    batch = BatchedAnts(gen.cfg, E, device=local_rank, evap_mode=args.evap, rng_seed=20261018, env_id_base=rank * E,
-                        record=record)
-    batch.import_state(stack_states(states, gen.cfg["reward_kind"]))
-    del states
-    batch.activate_all_pheromones(np.ones((E, N, wl["n_phero"])) * 10.0)      # agent.initialize, collect_agent.py:100
+    gen, batch, record, rot_tape, ph_tape = make_batch(args, rank, local_rank)
     C = len(gen.cfg["channels"])
-    rs = np.random.RandomState(12345 + rank)
-    n_tape = max(K, 32)                                                       # the pre-recorded action sequence
-    rot_tape = torch.from_numpy((rs.randint(0, 3, size=(n_tape, E, N)) - 1).astype(np.int8)).cuda()
-    ph_tape = torch.from_numpy(rs.randint(0, 3, size=(n_tape, E, N)).astype(np.int8)).cuda()
-    batch.observe()                                                           # main.py:88
+    n_tape = rot_tape.shape[0]
     t_setup = time.perf_counter() - t_setup
     episode_step = [0]
+    last_outputs = [None]                  # (obs, agent_state, reward) of the latest step, device tensors
 
     def run_steps(n):
         """n x [step(actions_t); update()] as C calls over the device-resident tape (ants_rollout: no Python, no host
@@ -304,7 +350,7 @@ def run_ours(args):
         done = 0
         while done < n:
             m = min(n_tape, n - done)
-            batch.rollout(rot_tape[:m], ph_tape[:m])
+            last_outputs[0] = batch.rollout(rot_tape[:m], ph_tape[:m])
             done += m
         episode_step[0] += n
 
@@ -335,6 +381,8 @@ def run_ours(args):
         ms = timed(K)
     launches = batch.stats()["kernel_launches"] - launches0
     value = world * E * N * K / (ms / 1000.0)
+    # the outputs of the last timed step, taken before the steps below overwrite them
+    dumped = sample_outputs(*last_outputs[0]) if args.dump_outputs and rank == 0 else None
 
     # ---- per-kernel timing (the following K steps, CUDA events around every launch on the launching stream)
     batch.set_profiling(True)
@@ -441,6 +489,9 @@ def run_ours(args):
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         cpu = run_cpu_baseline(wl, 3, args.cpu_steps)
+
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
 
     if rank == 0:
         line = {
@@ -576,13 +627,7 @@ def emit(line):
         os.write(_REAL_STDOUT, data)
 
 
-def main():
-    # Libraries print on fd 1 (NCCL's version banner comes from C, whatever NCCL_DEBUG says): everything but the
-    # final JSON line is sent to stderr.
-    global _REAL_STDOUT
-    sys.stdout.flush()
-    _REAL_STDOUT = os.dup(1)
-    os.dup2(2, 1)
+def make_parser():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=200)
@@ -599,7 +644,23 @@ def main():
     ap.add_argument("--late-start", type=int, default=900,
                     help="episode step at which the K steps are timed again (0 = skip the late window)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them returned (obs, agent_state, reward; rank "
+                         "0's envs) as DIR/<name>.npy, at most 64 MB: a fixed sample of the ants when all do not fit")
+    return ap
+
+
+def main():
+    # Libraries print on fd 1 (NCCL's version banner comes from C, whatever NCCL_DEBUG says): everything but the
+    # final JSON line is sent to stderr.
+    global _REAL_STDOUT
+    sys.stdout.flush()
+    _REAL_STDOUT = os.dup(1)
+    os.dup2(2, 1)
+    ap = make_parser()
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "cfg1"):
+        ap.error("--dump-outputs writes the outputs of the GPU step loop (--impl ours, workload cfg2/cfg3/cfg4)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "ours" and args.gpus > 1 and "WORLD_SIZE" not in os.environ:

@@ -71,6 +71,16 @@ def run_reference(cfg, init, tape):
     return rec
 
 
+def save_npz(path, arrays):
+    """np.savez with bzip2-compressed members (np.load reads them): the per-step observations of a scenario compress
+    to well under 1 MB this way, about a third smaller than with np.savez_compressed."""
+    import zipfile
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_BZIP2, compresslevel=9) as zf:
+        for k, v in arrays.items():
+            with zf.open(k + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asanyarray(v), allow_pickle=False)
+
+
 def main():
     only = set(sys.argv[1:])
     for name, kw in GOLDEN_SCENARIOS:
@@ -85,7 +95,7 @@ def main():
             out["tape_" + k] = np.asarray(v)
         out.update(rec)
         path = os.path.join(HERE, name + ".npz")
-        np.savez_compressed(path, **out)
+        save_npz(path, out)
         print("%-18s T=%3d hits=%4d anthill_food=%6.1f explored=%6d  %7.1f KB" % (
             name, tape["rot"].shape[0], int(rec["wall_hits"]), float(rec["final_anthill_food"]),
             int(rec["final_explored"].sum()), os.path.getsize(path) / 1024))

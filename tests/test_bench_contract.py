@@ -1,10 +1,13 @@
 """bench.py's contract, as far as it can be checked without a GPU: the reference arm (`--impl reference`, the
 reference algorithm on the host cores) prints ONE JSON line with the contract's keys, ranks other than 0 stay silent,
-and the algorithmic-byte accounting matches SURVEY.md section 8-d / DESIGN.md section 3."""
+and the algorithmic-byte accounting matches SURVEY.md section 8-d / DESIGN.md section 3.  On a GPU: `--dump-outputs`
+writes the same outputs in two runs with the same arguments."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -61,6 +64,72 @@ def test_algorithmic_bytes_follow_the_survey():
     assert abs(fused - step) < 1e-9
     peak, src = bench.load_peaks()
     assert 5000 < peak < 9000 and ("measured" in src or "fallback" in src)
+
+
+def test_dump_outputs_sample_is_fixed_and_bounded(monkeypatch):
+    """--dump-outputs: every ant while they fit, else the documented seeded sample of rows, the same rows in every array;
+    obs / agent_state stay f32 and reward f64."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    rs = np.random.RandomState(1)
+    E, N, S, C = 3, 40, 7, 6
+    obs = torch.from_numpy(rs.random_sample((E, N, S, S, C)).astype(np.float32))
+    ast = torch.from_numpy(rs.random_sample((E, N, 2)).astype(np.float32))
+    rew = torch.from_numpy(rs.random_sample((E, N)))
+    full = bench.sample_outputs(obs, ast, rew)
+    assert np.array_equal(full["obs"], obs.numpy().reshape(E * N, S, S, C))
+    assert np.array_equal(full["agent_state"], ast.numpy().reshape(E * N, 2))
+    assert np.array_equal(full["reward"], rew.numpy().reshape(E * N))
+    per_ant = S * S * C * 4 + 2 * 4 + 8
+    monkeypatch.setattr(bench, "DUMP_BYTES", 3 * 4096 + 50 * per_ant)
+    part = bench.sample_outputs(obs, ast, rew)
+    rows = np.sort(np.random.RandomState(0).choice(E * N, 50, replace=False))
+    assert part["obs"].dtype == np.float32 and part["agent_state"].dtype == np.float32 and part["reward"].dtype == np.float64
+    assert np.array_equal(part["obs"], full["obs"][rows]) and np.array_equal(part["agent_state"], full["agent_state"][rows])
+    assert np.array_equal(part["reward"], full["reward"][rows])
+    assert sum(a.nbytes for a in part.values()) <= bench.DUMP_BYTES
+
+
+def test_dump_outputs_is_refused_where_there_is_no_gpu_step_loop():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", "x"],
+                       capture_output=True, text=True, cwd=ROOT, timeout=600)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and r.stdout == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_those_of_the_last_timed_step(tmp_path):
+    """Two runs with the same arguments time exactly --steps steps and write the same outputs; they are the outputs of
+    the last timed step: the same inputs driven here through the warm-up and timed rollouts give them again."""
+    import numpy as np
+    args = ["--workload", "cfg2", "--envs", "16", "--steps", "7", "--warmup", "3", "--late-start", "0", "--e2e-steps", "0",
+            "--no-cpu-baseline"]
+    for k in range(2):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args, "--dump-outputs", str(tmp_path / str(k))],
+                           capture_output=True, text=True, cwd=ROOT, timeout=900)
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads(r.stdout)
+        assert d["steps"] == 7 and d["config"]["timed_steps"].startswith("steps 3-10 ")
+    names = ("agent_state", "obs", "reward")
+    assert sorted(os.listdir(tmp_path / "0")) == [n + ".npy" for n in names]
+    got = [{n: np.load(str(tmp_path / str(k) / (n + ".npy"))) for n in names} for k in range(2)]
+    assert got[0]["obs"].shape == (16 * 50, 7, 7, 6) and got[0]["obs"].dtype == np.float32
+    assert got[0]["agent_state"].shape == (16 * 50, 2) and got[0]["reward"].shape == (16 * 50,)
+    assert got[0]["reward"].dtype == np.float64 and np.abs(got[0]["obs"]).sum() > 0
+    for n in names:
+        assert np.array_equal(got[0][n], got[1][n]), n
+    sys.path.insert(0, ROOT)
+    import bench
+    a = bench.make_parser().parse_args(args)
+    _, batch, _, rot, ph = bench.make_batch(a)
+    try:
+        batch.rollout(rot[:a.warmup], ph[:a.warmup])
+        want = bench.sample_outputs(*batch.rollout(rot[:a.steps], ph[:a.steps]))
+    finally:
+        batch.close()
+    for n in names:
+        assert np.array_equal(got[0][n], want[n]), n
 
 
 def test_hand_typed_multi_gpu_run_becomes_the_torchrun_launch():
