@@ -1436,6 +1436,9 @@ __global__ void k_lazy_fold(Params p, uint32_t now, uint32_t now_abs, int unbox)
             // written as a plain number valid at timestamp 0 (never re-boxed: it is no longer max_val unless age 0)
             if (p.rec16) reinterpret_cast<float *>(r)[k] = (float)v; else reinterpret_cast<double *>(r)[k] = v;
             rec_set_ts(p, r, k, 0u);
+            // an unboxed deposit is a plain value like any other: the row perception kernel decodes plain values and
+            // later folds re-base them only while the flag is set
+            if (boxed && v != 0.0 && *p.plain_flag == 0u) *p.plain_flag = 1u;
         }
     }
 }

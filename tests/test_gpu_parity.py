@@ -195,8 +195,10 @@ def test_odd_configurations(name, kw, evap_mode):
 
 
 def test_lazy_timestamp_fold():
-    """More updates than the 12-bit timestamp range: the fold pass keeps the lazily decayed field equal to the
-    eagerly evaporated one (compared between two handles of the CUDA path itself, 4200 updates)."""
+    """More updates than the 12-bit timestamp range with float activations: every deposit saturates, so the field holds
+    boxed deposits only and the fold passes return at once.  Checks those boxed deposits against the eagerly evaporated
+    field (two handles of the CUDA path itself, 4200 updates); the fold's plain-value branches are covered by
+    tests/test_gpu_handle_age.py."""
     import torch
     from antsrl_b200 import BatchedAnts
     cfg, init, tape = make_scenario(seed=41, w=32, h=32, n_ants=16, steps=8)
