@@ -19,7 +19,7 @@ EXPORTED_SYMBOLS = [
     "ants_update", "ants_rollout", "ants_host_alloc", "ants_host_free", "ants_observe_host", "ants_step_host",
     "ants_update_host", "ants_get_stats", "ants_set_profiling", "ants_get_kernel_ms", "ants_reset_kernel_ms",
     "ants_sample_actions", "ants_export_env_state", "ants_packed_layout", "ants_step_host_packed", "ants_unpack_obs",
-    "ants_import_env_state",
+    "ants_import_env_state", "ants_generate_env_maps",
 ]
 
 

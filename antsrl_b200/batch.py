@@ -23,7 +23,7 @@ DEFAULT_MASK = np.array([[0, 0, 1, 1, 1, 0, 0],
 _REWARD_KINDS = {"all": _cabi.REWARD_ALL, "explore": _cabi.REWARD_EXPLORE, "food": _cabi.REWARD_FOOD}
 _EVAP_MODES = {"dense": _cabi.EVAP_DENSE, "tiles": _cabi.EVAP_ACTIVE_TILES, "lazy": _cabi.EVAP_LAZY}
 KERNEL_FAMILIES = ("move", "food_commit", "perceive", "collide", "rocks", "evaporate", "deposit", "absorb", "misc",
-                   "env_move", "env_update", "env_update_move", "pack")
+                   "env_move", "env_update", "env_update_move", "pack", "reset")
 
 
 def make_config(w, h, n_ants, n_phero=2, n_rocks=0, max_time=1000, radius=3, mask="default", fwd_delta=4,
@@ -117,6 +117,7 @@ class BatchedAnts:
         self.S = 2 * cfg["radius"] + 1
         self.C = len(cfg["channels"])
         self.device = torch.device("cuda", device)
+        self.env_id_base = int(env_id_base)          # global id of env 0 (sharding: seeds, Philox streams)
         self._c_cfg = build_c_config(cfg, n_envs, device, evap_mode, rng_seed, env_id_base, record=record)
         h = C.c_void_p()
         check(self.lib, self.lib.ants_create(C.byref(self._c_cfg), C.byref(h)))
@@ -180,6 +181,23 @@ class BatchedAnts:
         hs.rw_alias = (1 if state["rw_alias"] else 0) if state.get("rw_alias") is not None else -1
         hs.act_bool = (1 if state["act_bool"] else 0) if state.get("act_bool") is not None else -1
         check(self.lib, self.lib.ants_import_env_state(self._h, env0, n_envs, C.byref(hs)))
+
+    def generate_env_maps(self, anthill_xyr, wall_discs, food_discs, envs=None):
+        """ants_generate_env_maps: new maps for all envs, or with ``envs=(env0, n)`` for that window, written on the
+        device from the discs of CirclesGenerator maps: anthill_xyr (n, 3), wall_discs (n, Kw, 3), food_discs (n, Kf, 3)
+        int arrays of (xc, yc, r).  Pheromones, explored and occupancy are cleared; ants, rocks, the anthill store and
+        the batch scalars are left to :meth:`import_state`."""
+        env0, n_envs = (0, self.E) if envs is None else (int(envs[0]), int(envs[1]))
+        hill = np.ascontiguousarray(anthill_xyr, dtype=np.int32)
+        wd = np.ascontiguousarray(wall_discs, dtype=np.int32)
+        fd = np.ascontiguousarray(food_discs, dtype=np.int32)
+        if hill.shape != (n_envs, 3) or wd.ndim != 3 or wd.shape[0] != n_envs or wd.shape[2] != 3 \
+                or fd.ndim != 3 or fd.shape[0] != n_envs or fd.shape[2] != 3:
+            raise ValueError("expected anthill_xyr (%d, 3), wall_discs and food_discs (%d, K, 3); got %r, %r, %r"
+                             % (n_envs, n_envs, hill.shape, wd.shape, fd.shape))
+        i32 = C.POINTER(C.c_int32)
+        check(self.lib, self.lib.ants_generate_env_maps(self._h, env0, n_envs, hill.ctypes.data_as(i32), int(wd.shape[1]),
+                                                        wd.ctypes.data_as(i32), int(fd.shape[1]), fd.ctypes.data_as(i32)))
 
     def export_state(self, keys=None, envs=None):
         """The state dict of the whole batch, or with ``envs=(env0, n)`` of that window of environments only

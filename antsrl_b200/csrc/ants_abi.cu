@@ -4,6 +4,7 @@
 // arrays and the pitched HBM layout.
 #include "../../include/antsrl_b200.h"
 #include "ants_kernels.cuh"
+#include "ants_reset.cuh"
 #include "ants_pack.cuh"
 #include "ants_host_unpack.h"
 
@@ -45,9 +46,10 @@ int fail(int code, const char *fmt, ...) {
     } while (0)
 
 enum Fam { F_MOVE = 0, F_FOOD, F_PERCEIVE, F_COLLIDE, F_ROCKS, F_EVAP, F_DEPOSIT, F_ABSORB, F_MISC, F_ENV_MOVE, F_ENV_UPDATE,
-           F_ENV_FUSED, F_PACK, F_COUNT };
+           F_ENV_FUSED, F_PACK, F_RESET, F_COUNT };
 const char *kFamName[F_COUNT] = {"move", "food_commit", "perceive", "collide", "rocks", "evaporate",
-                                 "deposit", "absorb", "misc", "env_move", "env_update", "env_update_move", "pack"};
+                                 "deposit", "absorb", "misc", "env_move", "env_update", "env_update_move", "pack",
+                                 "reset"};
 
 struct TimedLaunch {
     cudaEvent_t a, b;
@@ -219,6 +221,9 @@ struct AntsBatch {
     int grouped = 0;                // inside a grouped rollout (whole-batch passes must join the groups first)
     cudaStream_t cur_stream = nullptr;   // target of the step-kernel launches: nullptr = the handle's stream, whole batch
     int cur_env0 = 0, cur_env1 = 0;
+    // ants_generate_env_maps: device copy of the window's discs (grows to the largest window seen, freed by ants_destroy)
+    int4 *reset_discs = nullptr;
+    int64_t reset_cap = 0;
 };
 
 namespace {
@@ -1245,6 +1250,7 @@ int ants_destroy(AntsBatch *b) {
     for (auto &g : b->groups) { if (g.s) { cudaStreamSynchronize(g.s); cudaStreamDestroy(g.s); } if (g.done) cudaEventDestroy(g.done); }
     if (b->ev_fork) cudaEventDestroy(b->ev_fork);
     if (b->h_packed) cudaFreeHost(b->h_packed);
+    if (b->reset_discs) cudaFree(b->reset_discs);
     for (auto e : b->chunk_ev) cudaEventDestroy(e);
     delete b->unpack_plan;
     if (b->own_stream) cudaStreamDestroy(b->own_stream);
@@ -1389,6 +1395,78 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
 int ants_import_state(AntsBatch *b, const AntsHostState *s) {
     if (!b) return fail(ANTS_E_ARG, "null argument");
     return ants_import_env_state(b, 0, b->p.E, s);
+}
+
+int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr, int32_t n_wall_discs,
+                           const int32_t *wall_discs, int32_t n_food_discs, const int32_t *food_discs) {
+    if (!b || !anthill_xyr) return fail(ANTS_E_ARG, "null argument");
+    Params &p = b->p;
+    if (env0 < 0 || n_envs < 1 || (int64_t)env0 + n_envs > p.E)
+        return fail(ANTS_E_ARG, "env window [%d, %d) outside the batch of %d envs", env0, env0 + n_envs, p.E);
+    if (n_wall_discs < 0 || n_food_discs < 0) return fail(ANTS_E_ARG, "negative disc count");
+    if ((n_wall_discs > 0 && !wall_discs) || (n_food_discs > 0 && !food_discs)) return fail(ANTS_E_ARG, "null disc array");
+    for (int e = 0; e < n_envs; ++e)
+        if (anthill_xyr[3 * e + 2] < 0) return fail(ANTS_E_ARG, "env %d: negative anthill radius", env0 + e);
+    // the discs of env e as (xc, yc, r, 0): its wall discs, then its food discs; each must lie inside the map
+    const int K = n_wall_discs + n_food_discs;
+    std::vector<int4> discs((size_t)n_envs * K);
+    for (int e = 0; e < n_envs; ++e)
+        for (int k = 0; k < K; ++k) {
+            const int32_t *d = k < n_wall_discs ? wall_discs + ((size_t)e * n_wall_discs + k) * 3
+                                                : food_discs + ((size_t)e * n_food_discs + (k - n_wall_discs)) * 3;
+            if (d[2] < 0 || d[0] - d[2] < 0 || d[0] + d[2] >= p.W || d[1] - d[2] < 0 || d[1] + d[2] >= p.H)
+                return fail(ANTS_E_ARG, "env %d: %s disc %d (%d, %d, r %d) does not lie inside the %d x %d map", env0 + e,
+                            k < n_wall_discs ? "wall" : "food", k < n_wall_discs ? k : k - n_wall_discs, d[0], d[1], d[2],
+                            p.W, p.H);
+            discs[(size_t)e * K + k] = make_int4(d[0], d[1], d[2], 0);
+        }
+    CK(cudaSetDevice(b->cfg.device));
+    cudaStream_t st = b->stream;
+    const bool whole = n_envs == p.E;
+    if ((int64_t)discs.size() > b->reset_cap) {
+        CK(cudaStreamSynchronize(st));                      // (the old buffer may still be read by an earlier launch)
+        if (b->reset_discs) { cudaFree(b->reset_discs); b->reset_discs = nullptr; b->reset_cap = 0; }
+        cudaError_t me = cudaMalloc(&b->reset_discs, discs.size() * sizeof(int4));
+        if (me != cudaSuccess) { b->reset_discs = nullptr; return fail(ANTS_E_ALLOC, "disc buffer: %s", cudaGetErrorString(me)); }
+        b->reset_cap = (int64_t)discs.size();
+    }
+    if (!discs.empty())
+        CK(cudaMemcpyAsync(b->reset_discs, discs.data(), discs.size() * sizeof(int4), cudaMemcpyHostToDevice, st));
+    std::vector<int32_t> hill4((size_t)n_envs * 4);
+    for (int e = 0; e < n_envs; ++e) {
+        const int32_t r = anthill_xyr[3 * e + 2];
+        hill4[4 * e] = anthill_xyr[3 * e]; hill4[4 * e + 1] = anthill_xyr[3 * e + 1];
+        hill4[4 * e + 2] = r; hill4[4 * e + 3] = r * r;
+    }
+    CK(cudaMemcpyAsync(p.hill + (size_t)env0 * 4, hill4.data(), hill4.size() * 4, cudaMemcpyHostToDevice, st));
+    ants::ResetArgs a;
+    a.discs = b->reset_discs; a.kw = n_wall_discs; a.kf = n_food_discs; a.env0 = env0;
+    a.tiles_x = (int)cdiv(p.Wp, ants::kResetTile); a.tiles_y = (int)cdiv(p.Hp, ants::kResetTile);
+    const unsigned grid = (unsigned)((int64_t)n_envs * a.tiles_x * a.tiles_y);
+    {
+        LaunchScope ls(b, F_RESET);
+        switch (p.rec_shift) {
+            case 3: ants::k_reset_maps<8><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
+            case 4: ants::k_reset_maps<16><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
+            case 5: ants::k_reset_maps<32><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
+            default: ants::k_reset_maps<64><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
+        }
+    }
+    TRY(check_launch("k_reset_maps"));
+    if (p.tile_active)
+        CK(cudaMemsetAsync(p.tile_active + (size_t)env0 * p.tiles_x * p.tiles_y, 0, (size_t)n_envs * p.tiles_x * p.tiles_y, st));
+    // the same bookkeeping as an import of food, walls, explored, pheromones and the anthill (ants_import_env_state)
+    if (p.owner) CK(cudaMemsetAsync(p.owner, 0, (size_t)p.E * p.plane * sizeof(uint32_t), st));
+    if (b->fused) CK(cudaMemsetAsync(p.absorb_count + env0, 0, (size_t)n_envs * sizeof(uint32_t), st));
+    else if (whole) CK(cudaMemsetAsync(p.absorb_count, 0, 2 * sizeof(uint32_t), st));
+    b->needs_sweep = 1;                                     // food may lie inside the new anthill disc (Q10)
+    b->move_done = 0;
+    b->pack_disabled = 0;
+    b->wall_flags_valid = 0;
+    b->owner_phase = 0;
+    if (whole) { b->obs_gen = 0; b->occ_gen = 0; }
+    CK(cudaStreamSynchronize(st));   // host temporaries above must outlive the copies
+    return ANTS_OK;
 }
 
 int ants_export_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, AntsHostState *s) {

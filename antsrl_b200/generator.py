@@ -35,13 +35,22 @@ class CirclesGenerator:
             self._stamps[r] = d[:, None] ** 2 + d[None, :] ** 2 <= r * r
         return self._stamps[r]
 
-    def generate(self, w, h):
-        gen = np.zeros((w, h), dtype=bool)
-        for _ in range(self.n_circles):
+    def draw_discs(self, w, h):
+        """-> int32 (n_circles, 3) array of (xc, yc, r): exactly the `random.random()` calls of `generate`, in its order.
+        Every disc lies inside the map (xc - r >= 0, xc + r < w, same for y) whenever w, h > 2 * max_radius, up to a
+        draw rounding to the upper end; `disc_inside` tells."""
+        out = np.empty((self.n_circles, 3), dtype=np.int32)
+        for i in range(self.n_circles):
             radius = int(random.random() * (self.max_radius - self.min_radius) + self.min_radius)
             xc = int(random.random() * (w - 2 * radius) + radius)
             yc = int(random.random() * (h - 2 * radius) + radius)
-            # the reference indexes gen[x, y] for x in [xc - r, xc + r]; numpy wraps negative indices
+            out[i] = (xc, yc, radius)
+        return out
+
+    def stamp(self, w, h, discs):
+        """bool (w, h): the union of the discs, with the reference's indexing (gen[x, y] for x in [xc - r, xc + r])."""
+        gen = np.zeros((w, h), dtype=bool)
+        for xc, yc, radius in np.asarray(discs).tolist():
             xi = np.arange(xc - radius, xc + radius + 1)
             yi = np.arange(yc - radius, yc + radius + 1)
             if xi[0] >= 0 and xi[-1] < w and yi[0] >= 0 and yi[-1] < h:
@@ -53,6 +62,16 @@ class CirclesGenerator:
                         if st[a, b]:
                             gen[x, y] = True
         return gen
+
+    def generate(self, w, h):
+        return self.stamp(w, h, self.draw_discs(w, h))
+
+
+def disc_inside(discs, w, h):
+    """True iff every (xc, yc, r) disc has r >= 0 and lies inside the w x h map (what ants_generate_env_maps takes)."""
+    d = np.asarray(discs, dtype=np.int64).reshape(-1, 3)
+    return bool(np.all((d[:, 2] >= 0) & (d[:, 0] - d[:, 2] >= 0) & (d[:, 0] + d[:, 2] < w) &
+                       (d[:, 1] - d[:, 2] >= 0) & (d[:, 1] + d[:, 2] < h)))
 
 
 from .perlin import PerlinGenerator   # noqa: E402,F401  (map_generators.py:9-25; parity unpinned, see perlin.py)
@@ -110,10 +129,57 @@ def stack_states(states, reward_kind="all"):
         else:
             out[k] = np.stack([np.asarray(s[k]) for s in states])
     if reward_kind == "all" and "rw_prev_dist" not in out:      # reward_custom.py:77
-        ax = out["anthill_xyr"][:, 0:1].astype(float)
-        ay = out["anthill_xyr"][:, 1:2].astype(float)
-        out["rw_prev_dist"] = ((out["x"] - ax) ** 2 + (out["y"] - ay) ** 2) ** 0.5
+        out["rw_prev_dist"] = _prev_dist(out["x"], out["y"], out["anthill_xyr"])
     return out
+
+
+def _prev_dist(x, y, anthill_xyr):
+    """All_Rewards' initial distance to the anthill (reward_custom.py:77), the rule of stack_states."""
+    ax = np.asarray(anthill_xyr)[..., 0:1].astype(float)
+    ay = np.asarray(anthill_xyr)[..., 1:2].astype(float)
+    return ((x - ax) ** 2 + (y - ay) ** 2) ** 0.5
+
+
+def generate_episode(w, h, n_ants, n_pheromones, n_rocks, food_generator, walls_generator, seed=None, max_hold=5,
+                     draw_ant_seed=True):
+    """The random draws of `generate_state` with the same arguments, from the global RNGs in the same order, without
+    the planes: a dict of anthill_xyr (3,), wall_discs / food_discs (n, 3) int32, the rocks, the ants' x, y, theta,
+    seed and rw_prev_dist.  -> None when the episode has no disc form (a generator that is not a CirclesGenerator:
+    nothing is drawn then; or a disc that does not lie inside the map): `generate_state` builds such maps."""
+    if type(food_generator) is not CirclesGenerator or type(walls_generator) is not CirclesGenerator:
+        return None
+    if seed is not None:
+        random.seed(seed)
+        np.random.seed(seed * 5)
+    m = min(w, h)
+    ax = int(random.random() * w * 0.5 + w * 0.25)
+    ay = int(random.random() * h * 0.5 + h * 0.25)
+    ar = int(random.random() * m * 0.05 + m * 0.05)
+    ep = {"anthill_xyr": np.array([ax, ay, ar], dtype=np.int32), "wall_discs": walls_generator.draw_discs(w, h),
+          "food_discs": food_generator.draw_discs(w, h)}
+    if n_rocks > 0:   # generate_state's draws, same order
+        c = np.random.random((n_rocks, 2))
+        c[:, 0] *= w * 0.75
+        c[:, 1] *= h * 0.25
+        c[:, 0] += w * 0.25
+        c[:, 1] += h * 0.25
+        ep["rock_centers"] = c
+        ep["rock_radii"] = np.random.random(n_rocks) * 5 + 5
+        ep["rock_weights"] = np.random.random(n_rocks) * 50 + 50
+    ang = np.random.random(n_ants) * 2 * np.pi
+    dist = np.random.random(n_ants) * ar * 0.8
+    x = np.cos(ang) * dist + ax
+    y = np.sin(ang) * dist + ay
+    t = np.random.random(n_ants) * 2 * np.pi
+    ep["x"] = np.mod(x, w)
+    ep["y"] = np.mod(y, h)
+    ep["theta"] = t
+    if draw_ant_seed:
+        ep["seed"] = np.random.random(n_ants)
+    ep["rw_prev_dist"] = _prev_dist(ep["x"], ep["y"], ep["anthill_xyr"])
+    if not (disc_inside(ep["wall_discs"], w, h) and disc_inside(ep["food_discs"], w, h)):
+        return None
+    return ep
 
 
 class BatchedEnvironmentGenerator:
@@ -146,3 +212,55 @@ class BatchedEnvironmentGenerator:
         if float_activation and self.n_pheromones > 0:   # what agent.initialize does, collect_agent.py:100-102
             batch.activate_all_pheromones(np.ones((n_envs, self.n_ants, self.n_pheromones)) * 10.0)
         return batch
+
+    def reset(self, batch, seed_base, envs=None, float_activation=True):
+        """A new episode for every env of `batch` (a BatchedAnts of this configuration), or with ``envs=(env0, n)`` for
+        that window only (main.py:66-79 generates a new environment per episode).  Env e gets the episode drawn with
+        seed ``seed_base + batch.env_id_base + e`` (its global id, as in `generate`), and the handle ends up in the state
+        `generate` would build from those seeds; a window reset keeps the batch's timestep and flags (lockstep).
+
+        With CirclesGenerator walls and food whose discs all lie inside the map, only the draws are made on the host
+        (`generate_episode`) and the maps are written on the device (`BatchedAnts.generate_env_maps`); otherwise (Perlin
+        walls, a duck-typed generator, a map smaller than a disc) the complete state is built on the host and imported.
+        Both give the same result.  -> "device" or "host", the path taken."""
+        env0, n = (0, batch.E) if envs is None else (int(envs[0]), int(envs[1]))
+        if env0 < 0 or n < 1 or env0 + n > batch.E:
+            raise ValueError("env window (%d, %d) outside the batch of %d envs" % (env0, n, batch.E))
+        seeds = [seed_base + batch.env_id_base + env0 + e for e in range(n)]
+        args = (self.w, self.h, self.n_ants, self.n_pheromones, self.n_rocks, self.food_generator, self.walls_generator)
+        eps = []
+        for s in seeds:
+            ep = generate_episode(*args, seed=s)
+            if ep is None:
+                break
+            eps.append(ep)
+        N, P = self.n_ants, self.n_pheromones
+        if len(eps) == n:
+            path = "device"
+            batch.generate_env_maps(np.stack([ep["anthill_xyr"] for ep in eps]), np.stack([ep["wall_discs"] for ep in eps]),
+                                    np.stack([ep["food_discs"] for ep in eps]), envs=(env0, n))
+            keys = ("x", "y", "theta", "seed", "rw_prev_dist") + (("rock_centers", "rock_radii", "rock_weights")
+                                                                  if self.n_rocks > 0 else ())
+            st = {k: np.stack([ep[k] for ep in eps]) for k in keys}
+        else:
+            path = "host"
+            st = stack_states([generate_state(*args, seed=s) for s in seeds], "all")
+            for k in ("act_bool", "rw_alias", "timestep"):
+                st.pop(k)
+            st["phero"] = np.zeros((n, P, self.w, self.h))
+            st["explored"] = np.zeros((n, self.w, self.h), dtype=np.uint8)
+        # the per-ant state of a new episode (Ants.__init__, All_Rewards.__init__), the anthill store emptied
+        if self.cfg["reward_kind"] != "all":
+            st["rw_prev_dist"] = np.zeros((n, N))        # (generate() leaves it as a new handle has it)
+        st["prev_x"], st["prev_y"], st["prev_theta"] = st["x"], st["y"], st["theta"]
+        for k in ("holding", "rewards", "rw_holding_prev"):
+            st[k] = np.zeros((n, N))
+        st["mandibles"] = np.zeros((n, N), dtype=np.uint8)
+        st["reward_state"] = np.zeros((n, N), dtype=np.uint8)
+        st["anthill_food"] = np.zeros(n)
+        floats = float_activation and P > 0            # what agent.initialize does, collect_agent.py:100-102
+        st["activation"] = np.full((n, N, P), 10.0 if floats else 0.0)
+        if n == batch.E:
+            st["timestep"], st["rw_alias"], st["act_bool"] = 1, True, not floats
+        batch.import_state(st, envs=(env0, n))
+        return path

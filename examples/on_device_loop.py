@@ -6,7 +6,11 @@ observation -> epsilon-greedy action (a torch MLP with the collect agents' two h
 -> update, for E environments at once.  Observations, actions, rewards and the replay memory never cross PCIe; the
 only host traffic per step is kernel launches.  PyTorch is plumbing (the MLP and the ring-buffer copies).
 
-    python examples/on_device_loop.py [--envs 512] [--steps 50] [--workload cfg4]
+    python examples/on_device_loop.py [--envs 512] [--steps 50] [--workload cfg4] [--episodes K]
+
+With --episodes K > 1 an episode lasts --steps steps, and when `done` arrives every env starts a new one
+(main.py:66-79) through BatchedEnvironmentGenerator.reset, which writes the new maps on the device; the share of the
+wall time spent in those resets is printed.
 """
 import argparse
 import os
@@ -47,10 +51,11 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--epsilon", type=float, default=0.3)
     ap.add_argument("--replay", type=int, default=1 << 20)
+    ap.add_argument("--episodes", type=int, default=1, help="episodes of --steps steps each (1: one episode, no reset)")
     a = ap.parse_args()
     wl = bench.WORKLOADS[a.workload]
     E, N = a.envs, wl["n_ants"]
-    gen = bench.make_generator(wl, a.steps + 10)
+    gen = bench.make_generator(wl, a.steps + 10 if a.episodes <= 1 else a.steps)
     states = bench.generate_states_parallel(wl, a.steps + 10, 0, E)
     env = BatchedAnts(gen.cfg, E, evap_mode="lazy", record="compact8")
     env.import_state(stack_states(states, "all"))
@@ -63,7 +68,9 @@ def main():
     obs, ast = obs.clone(), ast.clone()
     total_reward = torch.zeros((), dtype=torch.float64, device="cuda")
     warm = 5                                                                     # cuBLAS / allocator warm-up, untimed
-    for t in range(a.steps + warm):
+    n_iter = a.steps + warm if a.episodes <= 1 else a.steps * a.episodes
+    reset_s, episode = 0.0, 0
+    for t in range(n_iter):
         if t == warm:
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -76,11 +83,22 @@ def main():
         env.update(None)                                                         # main.py:131
         total_reward += rew.sum()
         obs, ast = new_obs.clone(), new_ast.clone()
+        if done and a.episodes > 1 and episode + 1 < a.episodes:                # main.py:66-79: a new environment
+            episode += 1
+            r0 = time.perf_counter()
+            gen.reset(env, gen.seed_base + episode * E)                          # (reset synchronises the stream)
+            obs, ast, _, _ = env.observe()
+            obs, ast = obs.clone(), ast.clone()
+            torch.cuda.synchronize()
+            reset_s += time.perf_counter() - r0
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
+    n_steps = n_iter - warm
     print("on-device loop: %d envs x %d ants x %d steps in %.3f s = %.3e ant-steps/s (policy forward + replay ingest "
           "included), mean reward/ant-step %.4f, replay fill %d" %
-          (E, N, a.steps, dt, E * N * a.steps / dt, float(total_reward) / (E * N * a.steps), len(mem)))
+          (E, N, n_steps, dt, E * N * n_steps / dt, float(total_reward) / (E * N * n_steps), len(mem)))
+    if a.episodes > 1:
+        print("%d episodes: %d resets took %.3f s, %.1f %% of the wall time" % (episode + 1, episode, reset_s, 100.0 * reset_s / dt))
     env.close()
 
 

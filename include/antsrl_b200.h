@@ -152,6 +152,17 @@ int ants_export_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, AntsHostSt
 /* ... and the import of such a window: a new map / new ants for the envs [env0, env0 + n_envs) only (main.py:66-79
  * generates a new environment per episode), or a large batch uploaded in slices.  The scalars stay batch-wide. */
 int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const AntsHostState *s);
+/* A new episode's map for the envs [env0, env0 + n_envs), written on the device from the generator's random draws
+ * instead of dense planes (EnvironmentGenerator.generate, environment_generator.py:60-72, with CirclesGenerator walls
+ * and food).  Host arrays: anthill_xyr [n_envs][3], wall_discs [n_envs][n_wall_discs][3], food_discs
+ * [n_envs][n_food_discs][3] of (xc, yc, r).  A cell is a wall iff some wall disc has (x-xc)^2 + (y-yc)^2 <= r^2 and the
+ * cell lies outside the anthill disc; its food is 1.0 iff some food disc covers it and it is not a wall; pheromones,
+ * explored and occupancy are 0.  Afterwards the envs are in the state an import of food, walls, explored, pheromones
+ * and anthill leaves (the first update sweeps the anthill disc); the ants, rocks, anthill store and batch scalars are
+ * not touched: ants_import_env_state uploads those (kilobytes per env).  ANTS_E_ARG, with the handle unchanged, for a
+ * window outside the batch, a negative count or radius, or a disc that does not lie inside the map. */
+int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr, int32_t n_wall_discs,
+                           const int32_t *wall_discs, int32_t n_food_discs, const int32_t *food_discs);
 
 /* Ants.activate_all_pheromones, ants.py:86-87.  act: host [E][N][P] */
 int ants_activate_all_pheromones(AntsBatch *b, const double *act, int32_t is_bool);
@@ -222,7 +233,8 @@ int ants_unpack_obs(const AntsPackedLayout *layout, const void *h_packed, int64_
 int ants_get_stats(AntsBatch *b, AntsStats *out);
 /* time (ms) spent by the named kernel family since the last reset, measured with CUDA events on the handle's
  * stream when profiling is enabled with ants_set_profiling(b, 1): "perceive", "env_move", "env_update",
- * "env_update_move" (block-per-environment kernels), "evaporate", "absorb", "misc", "pack"; and for handles on the
+ * "env_update_move" (block-per-environment kernels), "evaporate", "absorb", "misc", "pack", "reset"
+ * (ants_generate_env_maps); and for handles on the
  * flat kernels (non-lazy field, > 1024 ants per env) "move", "food_commit", "collide", "rocks", "deposit" */
 int ants_set_profiling(AntsBatch *b, int32_t on);
 int ants_get_kernel_ms(AntsBatch *b, const char *name, double *ms, int64_t *launches);
