@@ -19,7 +19,7 @@ EXPORTED_SYMBOLS = [
     "ants_update", "ants_rollout", "ants_host_alloc", "ants_host_free", "ants_observe_host", "ants_step_host",
     "ants_update_host", "ants_get_stats", "ants_set_profiling", "ants_get_kernel_ms", "ants_reset_kernel_ms",
     "ants_sample_actions", "ants_export_env_state", "ants_packed_layout", "ants_step_host_packed", "ants_unpack_obs",
-    "ants_import_env_state", "ants_generate_env_maps",
+    "ants_import_env_state", "ants_generate_env_maps", "ants_generate_env_maps_ex", "ants_perlin_noise",
 ]
 
 
@@ -71,6 +71,12 @@ class AntsPackedLayout(C.Structure):
                 ("value_channel", C.c_int32 * 2), ("food_channel", C.c_int32), ("visible_index", C.c_uint8 * 228)]
 
 
+class AntsPerlinLayer(C.Structure):
+    _fields_ = [("offsets", C.POINTER(C.c_int32)), ("scale", C.c_double), ("density", C.c_double),
+                ("octaves", C.c_int32), ("reserved", C.c_int32), ("persistence", C.c_double),
+                ("lacunarity", C.c_double)]
+
+
 class AntsError(RuntimeError):
     pass
 
@@ -99,6 +105,9 @@ def load_library(path=None):
     lib.ants_export_state.argtypes = [vp, C.POINTER(AntsHostState)]
     lib.ants_export_env_state.argtypes = [vp, i32, i32, C.POINTER(AntsHostState)]
     lib.ants_import_env_state.argtypes = [vp, i32, i32, C.POINTER(AntsHostState)]
+    lib.ants_generate_env_maps_ex.argtypes = [vp, i32, i32, vp, i32, vp, C.POINTER(AntsPerlinLayer), i32, vp,
+                                              C.POINTER(AntsPerlinLayer)]
+    lib.ants_perlin_noise.argtypes = [i32, C.POINTER(AntsPerlinLayer), i32, i32, i32, vp, vp]
     lib.ants_activate_all_pheromones.argtypes = [vp, vp, i32]
     lib.ants_observe.argtypes = [vp, vp, vp, vp, vp]
     lib.ants_step.argtypes = [vp, vp, vp, vp, vp, vp, C.POINTER(i32)]

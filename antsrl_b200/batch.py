@@ -186,18 +186,35 @@ class BatchedAnts:
         """ants_generate_env_maps: new maps for all envs, or with ``envs=(env0, n)`` for that window, written on the
         device from the discs of CirclesGenerator maps: anthill_xyr (n, 3), wall_discs (n, Kw, 3), food_discs (n, Kf, 3)
         int arrays of (xc, yc, r).  Pheromones, explored and occupancy are cleared; ants, rocks, the anthill store and
-        the batch scalars are left to :meth:`import_state`."""
+        the batch scalars are left to :meth:`import_state`.
+
+        Either map argument may instead be a :class:`~antsrl_b200.perlin.PerlinLayer` (``PerlinGenerator.layer``: the
+        (n, 2) offsets of PerlinGenerator maps and the generator's parameters); that layer is then written from the
+        Perlin noise on the device (ants_generate_env_maps_ex), bit for bit as `PerlinGenerator.stamp`."""
+        from .perlin import PerlinLayer, perlin_layer_struct
         env0, n_envs = (0, self.E) if envs is None else (int(envs[0]), int(envs[1]))
         hill = np.ascontiguousarray(anthill_xyr, dtype=np.int32)
-        wd = np.ascontiguousarray(wall_discs, dtype=np.int32)
-        fd = np.ascontiguousarray(food_discs, dtype=np.int32)
+        keep, layers, discs = [], [], []
+        for what, m in (("wall", wall_discs), ("food", food_discs)):
+            if isinstance(m, PerlinLayer):
+                st, offs = perlin_layer_struct(m)
+                if offs.shape[0] != n_envs:
+                    raise ValueError("%s layer: expected the offsets of %d envs, got %r" % (what, n_envs, offs.shape))
+                keep.append(offs)
+                layers.append(C.pointer(st))
+                discs.append(np.zeros((n_envs, 0, 3), dtype=np.int32))
+            else:
+                layers.append(None)
+                discs.append(np.ascontiguousarray(m, dtype=np.int32))
+        wd, fd = discs
         if hill.shape != (n_envs, 3) or wd.ndim != 3 or wd.shape[0] != n_envs or wd.shape[2] != 3 \
                 or fd.ndim != 3 or fd.shape[0] != n_envs or fd.shape[2] != 3:
             raise ValueError("expected anthill_xyr (%d, 3), wall_discs and food_discs (%d, K, 3); got %r, %r, %r"
                              % (n_envs, n_envs, hill.shape, wd.shape, fd.shape))
         i32 = C.POINTER(C.c_int32)
-        check(self.lib, self.lib.ants_generate_env_maps(self._h, env0, n_envs, hill.ctypes.data_as(i32), int(wd.shape[1]),
-                                                        wd.ctypes.data_as(i32), int(fd.shape[1]), fd.ctypes.data_as(i32)))
+        check(self.lib, self.lib.ants_generate_env_maps_ex(self._h, env0, n_envs, hill.ctypes.data_as(i32),
+                                                           int(wd.shape[1]), wd.ctypes.data_as(i32), layers[0],
+                                                           int(fd.shape[1]), fd.ctypes.data_as(i32), layers[1]))
 
     def export_state(self, keys=None, envs=None):
         """The state dict of the whole batch, or with ``envs=(env0, n)`` of that window of environments only

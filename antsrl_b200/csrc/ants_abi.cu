@@ -9,6 +9,7 @@
 #include "ants_host_unpack.h"
 
 #include <math.h>
+#include <cmath>
 #include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
@@ -224,6 +225,9 @@ struct AntsBatch {
     // ants_generate_env_maps: device copy of the window's discs (grows to the largest window seen, freed by ants_destroy)
     int4 *reset_discs = nullptr;
     int64_t reset_cap = 0;
+    // ants_generate_env_maps_ex: device copy of the Perlin layers' offsets (the same lifetime)
+    int2 *reset_offsets = nullptr;
+    int64_t reset_offsets_cap = 0;
 };
 
 namespace {
@@ -1251,6 +1255,7 @@ int ants_destroy(AntsBatch *b) {
     if (b->ev_fork) cudaEventDestroy(b->ev_fork);
     if (b->h_packed) cudaFreeHost(b->h_packed);
     if (b->reset_discs) cudaFree(b->reset_discs);
+    if (b->reset_offsets) cudaFree(b->reset_offsets);
     for (auto e : b->chunk_ev) cudaEventDestroy(e);
     delete b->unpack_plan;
     if (b->own_stream) cudaStreamDestroy(b->own_stream);
@@ -1397,16 +1402,66 @@ int ants_import_state(AntsBatch *b, const AntsHostState *s) {
     return ants_import_env_state(b, 0, b->p.E, s);
 }
 
-int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr, int32_t n_wall_discs,
-                           const int32_t *wall_discs, int32_t n_food_discs, const int32_t *food_discs) {
+// Checks a Perlin layer of n envs on a W x H map (the ANTS_E_ARG cases of the header) and fills its device form, all
+// but the offsets pointer.  The checks keep every integer part of the noise inside int32, computed in float as pnoise2
+// computes: each octave's period 1024 * freq, and the scaled coordinates x' * freq of the map's edge cells, which bound
+// those of every cell because rounding is monotone (numpy silently casts NaN or out-of-range values to garbage).
+static int perlin_layer_check(const AntsPerlinLayer *L, int n, int W, int H, const char *what, ants::PerlinArgs *out) {
+    if (!L->offsets) return fail(ANTS_E_ARG, "%s: NULL offsets", what);
+    if (L->octaves < 1 || L->octaves > ants::kPerlinMaxOctaves)
+        return fail(ANTS_E_ARG, "%s: octaves %d outside 1 ... %d", what, L->octaves, ants::kPerlinMaxOctaves);
+    if (!std::isfinite(L->scale) || L->scale == 0.0) return fail(ANTS_E_ARG, "%s: scale %g", what, L->scale);
+    const float pers = (float)L->persistence, lac = (float)L->lacunarity;
+    if (!std::isfinite(pers) || !std::isfinite(lac))
+        return fail(ANTS_E_ARG, "%s: persistence %g or lacunarity %g is not a finite float", what, L->persistence,
+                    L->lacunarity);
+    const float lim = 2147483648.f;                          // 2^31
+    float freq[ants::kPerlinMaxOctaves];
+    freq[0] = 1.f;
+    for (int o = 0; o < L->octaves; ++o) {
+        if (o > 0) freq[o] = freq[o - 1] * lac;
+        const float rep = 1024.f * freq[o];
+        if (!(std::fabs(rep) < lim) || rep == 0.f)
+            return fail(ANTS_E_ARG, "%s: octave %d has the period %g (1024 * freq must be finite, non-zero, below 2^31)",
+                        what, o + 1, (double)rep);
+    }
+    for (int e = 0; e < n; ++e)
+        for (int c = 0; c < 4; ++c) {
+            const int64_t cell = (c & 1) ? (c < 2 ? W : H) - 1 : 0;
+            const float x = (float)((double)(cell + L->offsets[2 * e + (c >> 1)]) / L->scale);
+            for (int o = 0; o < L->octaves; ++o) {
+                const float xf = x * freq[o];
+                if (!(std::fabs(xf) < lim))
+                    return fail(ANTS_E_ARG, "%s: env %d, octave %d: the coordinate %g of a map edge is not finite or not "
+                                "below 2^31", what, e, o + 1, (double)xf);
+            }
+        }
+    out->offsets = nullptr;
+    out->scale = L->scale;
+    out->density = L->density;
+    out->octaves = L->octaves;
+    out->persistence = pers;
+    out->lacunarity = lac;
+    return ANTS_OK;
+}
+
+// ants_generate_env_maps and ants_generate_env_maps_ex (NULL Perlin layers: the former)
+static int generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr,
+                             int32_t n_wall_discs, const int32_t *wall_discs, const AntsPerlinLayer *wall_perlin,
+                             int32_t n_food_discs, const int32_t *food_discs, const AntsPerlinLayer *food_perlin) {
     if (!b || !anthill_xyr) return fail(ANTS_E_ARG, "null argument");
     Params &p = b->p;
     if (env0 < 0 || n_envs < 1 || (int64_t)env0 + n_envs > p.E)
         return fail(ANTS_E_ARG, "env window [%d, %d) outside the batch of %d envs", env0, env0 + n_envs, p.E);
     if (n_wall_discs < 0 || n_food_discs < 0) return fail(ANTS_E_ARG, "negative disc count");
     if ((n_wall_discs > 0 && !wall_discs) || (n_food_discs > 0 && !food_discs)) return fail(ANTS_E_ARG, "null disc array");
+    if ((wall_perlin && n_wall_discs != 0) || (food_perlin && n_food_discs != 0))
+        return fail(ANTS_E_ARG, "a layer given both discs and Perlin noise");
     for (int e = 0; e < n_envs; ++e)
         if (anthill_xyr[3 * e + 2] < 0) return fail(ANTS_E_ARG, "env %d: negative anthill radius", env0 + e);
+    ants::ResetPerlin pl = {};
+    if (wall_perlin) TRY(perlin_layer_check(wall_perlin, n_envs, p.W, p.H, "wall layer", &pl.wall));
+    if (food_perlin) TRY(perlin_layer_check(food_perlin, n_envs, p.W, p.H, "food layer", &pl.food));
     // the discs of env e as (xc, yc, r, 0): its wall discs, then its food discs; each must lie inside the map
     const int K = n_wall_discs + n_food_discs;
     std::vector<int4> discs((size_t)n_envs * K);
@@ -1420,6 +1475,11 @@ int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int
                             p.W, p.H);
             discs[(size_t)e * K + k] = make_int4(d[0], d[1], d[2], 0);
         }
+    // the offsets of the Perlin layers: the wall layer's n_envs pairs, then the food layer's
+    std::vector<int2> offs;
+    for (const AntsPerlinLayer *L : {wall_perlin, food_perlin})
+        if (L)
+            for (int e = 0; e < n_envs; ++e) offs.push_back(make_int2(L->offsets[2 * e], L->offsets[2 * e + 1]));
     CK(cudaSetDevice(b->cfg.device));
     cudaStream_t st = b->stream;
     const bool whole = n_envs == p.E;
@@ -1432,6 +1492,18 @@ int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int
     }
     if (!discs.empty())
         CK(cudaMemcpyAsync(b->reset_discs, discs.data(), discs.size() * sizeof(int4), cudaMemcpyHostToDevice, st));
+    if ((int64_t)offs.size() > b->reset_offsets_cap) {
+        CK(cudaStreamSynchronize(st));
+        if (b->reset_offsets) { cudaFree(b->reset_offsets); b->reset_offsets = nullptr; b->reset_offsets_cap = 0; }
+        cudaError_t me = cudaMalloc(&b->reset_offsets, offs.size() * sizeof(int2));
+        if (me != cudaSuccess) { b->reset_offsets = nullptr; return fail(ANTS_E_ALLOC, "offset buffer: %s", cudaGetErrorString(me)); }
+        b->reset_offsets_cap = (int64_t)offs.size();
+    }
+    if (!offs.empty()) {
+        CK(cudaMemcpyAsync(b->reset_offsets, offs.data(), offs.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
+        if (wall_perlin) pl.wall.offsets = b->reset_offsets;
+        if (food_perlin) pl.food.offsets = b->reset_offsets + (wall_perlin ? n_envs : 0);
+    }
     std::vector<int32_t> hill4((size_t)n_envs * 4);
     for (int e = 0; e < n_envs; ++e) {
         const int32_t r = anthill_xyr[3 * e + 2];
@@ -1445,11 +1517,20 @@ int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int
     const unsigned grid = (unsigned)((int64_t)n_envs * a.tiles_x * a.tiles_y);
     {
         LaunchScope ls(b, F_RESET);
-        switch (p.rec_shift) {
-            case 3: ants::k_reset_maps<8><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
-            case 4: ants::k_reset_maps<16><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
-            case 5: ants::k_reset_maps<32><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
-            default: ants::k_reset_maps<64><<<grid, ants::kResetThreads, 0, st>>>(p, a); break;
+        if (wall_perlin || food_perlin) {
+            switch (p.rec_shift) {
+                case 3: ants::k_reset_maps<8, true><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+                case 4: ants::k_reset_maps<16, true><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+                case 5: ants::k_reset_maps<32, true><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+                default: ants::k_reset_maps<64, true><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+            }
+        } else {
+            switch (p.rec_shift) {
+                case 3: ants::k_reset_maps<8><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+                case 4: ants::k_reset_maps<16><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+                case 5: ants::k_reset_maps<32><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+                default: ants::k_reset_maps<64><<<grid, ants::kResetThreads, 0, st>>>(p, a, pl); break;
+            }
         }
     }
     TRY(check_launch("k_reset_maps"));
@@ -1466,6 +1547,40 @@ int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int
     b->owner_phase = 0;
     if (whole) { b->obs_gen = 0; b->occ_gen = 0; }
     CK(cudaStreamSynchronize(st));   // host temporaries above must outlive the copies
+    return ANTS_OK;
+}
+
+int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr, int32_t n_wall_discs,
+                           const int32_t *wall_discs, int32_t n_food_discs, const int32_t *food_discs) {
+    return generate_env_maps(b, env0, n_envs, anthill_xyr, n_wall_discs, wall_discs, nullptr, n_food_discs, food_discs,
+                             nullptr);
+}
+
+int ants_generate_env_maps_ex(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr,
+                              int32_t n_wall_discs, const int32_t *wall_discs, const AntsPerlinLayer *wall_perlin,
+                              int32_t n_food_discs, const int32_t *food_discs, const AntsPerlinLayer *food_perlin) {
+    return generate_env_maps(b, env0, n_envs, anthill_xyr, n_wall_discs, wall_discs, wall_perlin, n_food_discs,
+                             food_discs, food_perlin);
+}
+
+int ants_perlin_noise(int32_t device, const AntsPerlinLayer *layer, int32_t n, int32_t w, int32_t h, float *d_out,
+                      void *stream) {
+    if (!layer || !d_out) return fail(ANTS_E_ARG, "null argument");
+    if (n < 1 || w < 1 || h < 1) return fail(ANTS_E_ARG, "empty field: n %d, w %d, h %d", n, w, h);
+    ants::PerlinArgs L;
+    TRY(perlin_layer_check(layer, n, w, h, "layer", &L));
+    const int tiles_x = (int)cdiv(w, ants::kPerlinTile), tiles_y = (int)cdiv(h, ants::kPerlinTile);
+    if ((int64_t)n * tiles_x * tiles_y > 0x7fffffff) return fail(ANTS_E_ARG, "field of %d x %d x %d too large", n, w, h);
+    CK(cudaSetDevice(device));
+    cudaStream_t st = (cudaStream_t)stream;
+    Scratch off;
+    CK(cudaMalloc(&off.ptr, (size_t)n * sizeof(int2)));
+    CK(cudaMemcpyAsync(off.ptr, layer->offsets, (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, st));
+    L.offsets = (const int2 *)off.ptr;
+    ants::k_perlin_field<<<(unsigned)((int64_t)n * tiles_x * tiles_y), ants::kPerlinThreads, 0, st>>>(
+        L, w, h, tiles_y, tiles_x * tiles_y, d_out);
+    TRY(check_launch("k_perlin_field"));
+    CK(cudaStreamSynchronize(st));   // the offsets buffer is freed on return
     return ANTS_OK;
 }
 

@@ -13,7 +13,13 @@
 // Empty pheromone fields and a 0 explored / occupancy stamp read the same under any lazy or generation counter, so the
 // host counters keep running.  8-byte records keep stale side-array slots: no code of the new map escapes to them.
 // With diffusion the current pheromone planes are zeroed too, with the wall bit in the sign (what k_plane_walls does).
+//
+// A layer may instead be Perlin noise (PerlinGenerator, the reference's default walls): the instantiation with PERLIN set
+// computes the noise of the tile's cells (ants_perlin.cuh, the function ants_perlin_noise uses too) and sets the layer's
+// bit where (double)noise > density; the disc list then holds the other layer's discs only.
 #pragma once
+
+#include "ants_perlin.cuh"
 
 namespace ants {
 
@@ -21,6 +27,7 @@ constexpr int kResetTile = 64;                 // cells per tile side (8 record 
 constexpr int kResetThreads = 256;
 constexpr int kResetChunk = 1024;              // discs culled per pass (the shared list holds at most one chunk)
 constexpr int kResetPairs = kResetTile * kResetTile / 2 / kResetThreads;   // record pairs per thread
+static_assert(kPerlinTile == kResetTile && kPerlinThreads == kResetThreads, "perlin_tile covers the reset tile");
 
 struct ResetArgs {
     const int4 *discs;      // [n_env][kw + kf] (xc, yc, r, 0): the wall discs of an env, then its food discs
@@ -28,6 +35,21 @@ struct ResetArgs {
     int32_t env0;           // first env of the window
     int32_t tiles_x, tiles_y;
 };
+
+struct ResetPerlin {        // Perlin layers of k_reset_maps<RB, true> (offsets NULL: the layer is discs)
+    PerlinArgs wall, food;
+};
+
+// sets bit k of `bits` where value k of the tile's noise exceeds the layer's density
+template <int PAIRS>
+__device__ __forceinline__ void perlin_layer_bits(PerlinSmem &s, const PerlinArgs &L, int el, int x0, int y0, int W,
+                                                  int H, uint32_t &bits) {
+    float v[2 * PAIRS];
+    perlin_tile<PAIRS>(s, L, el, x0, y0, W, H, v);
+#pragma unroll
+    for (int k = 0; k < 2 * PAIRS; ++k)
+        if ((double)v[k] > L.density) bits |= 1u << k;
+}
 
 // 64-bit word i of a record with the given fields (food 0 or 1); RB = record bytes
 template <int RB>
@@ -46,8 +68,8 @@ __device__ __forceinline__ unsigned long long reset_word(const Params &p, int i,
     return w;
 }
 
-template <int RB>
-__global__ void __launch_bounds__(kResetThreads) k_reset_maps(Params p, ResetArgs a) {
+template <int RB, bool PERLIN = false>
+__global__ void __launch_bounds__(kResetThreads) k_reset_maps(Params p, ResetArgs a, ResetPerlin pl) {
     __shared__ int4 list[kResetChunk];
     __shared__ int n_list;
     const int tiles = a.tiles_x * a.tiles_y;
@@ -94,6 +116,11 @@ __global__ void __launch_bounds__(kResetThreads) k_reset_maps(Params p, ResetArg
             }
         }
         __syncthreads();
+    }
+    if constexpr (PERLIN) {
+        __shared__ PerlinSmem ps;
+        if (pl.wall.offsets) perlin_layer_bits<kResetPairs>(ps, pl.wall, el, x0, y0, p.W, p.H, wall_bits);
+        if (pl.food.offsets) perlin_layer_bits<kResetPairs>(ps, pl.food, el, x0, y0, p.W, p.H, food_bits);
     }
 
     const int nbx = p.Wp >> 3;

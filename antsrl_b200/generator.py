@@ -141,13 +141,22 @@ def _prev_dist(x, y, anthill_xyr):
 
 
 def generate_episode(w, h, n_ants, n_pheromones, n_rocks, food_generator, walls_generator, seed=None, max_hold=5,
-                     draw_ant_seed=True):
+                     draw_ant_seed=True, perlin=False):
     """The random draws of `generate_state` with the same arguments, from the global RNGs in the same order, without
     the planes: a dict of anthill_xyr (3,), wall_discs / food_discs (n, 3) int32, the rocks, the ants' x, y, theta,
     seed and rw_prev_dist.  -> None when the episode has no disc form (a generator that is not a CirclesGenerator:
-    nothing is drawn then; or a disc that does not lie inside the map): `generate_state` builds such maps."""
-    if type(food_generator) is not CirclesGenerator or type(walls_generator) is not CirclesGenerator:
-        return None
+    nothing is drawn then; or a disc that does not lie inside the map): `generate_state` builds such maps.
+
+    With ``perlin=True`` a layer whose generator is exactly a `PerlinGenerator` has a draw form too: its two offsets,
+    returned as wall_perlin / food_perlin (2,) int32 instead of wall_discs / food_discs."""
+    kinds = []
+    for g in (walls_generator, food_generator):
+        if type(g) is CirclesGenerator:
+            kinds.append("discs")
+        elif perlin and type(g) is PerlinGenerator:
+            kinds.append("perlin")
+        else:
+            return None
     if seed is not None:
         random.seed(seed)
         np.random.seed(seed * 5)
@@ -155,8 +164,9 @@ def generate_episode(w, h, n_ants, n_pheromones, n_rocks, food_generator, walls_
     ax = int(random.random() * w * 0.5 + w * 0.25)
     ay = int(random.random() * h * 0.5 + h * 0.25)
     ar = int(random.random() * m * 0.05 + m * 0.05)
-    ep = {"anthill_xyr": np.array([ax, ay, ar], dtype=np.int32), "wall_discs": walls_generator.draw_discs(w, h),
-          "food_discs": food_generator.draw_discs(w, h)}
+    ep = {"anthill_xyr": np.array([ax, ay, ar], dtype=np.int32)}
+    for name, g, kind in (("wall", walls_generator, kinds[0]), ("food", food_generator, kinds[1])):   # walls first
+        ep[name + "_" + kind] = g.draw_discs(w, h) if kind == "discs" else g.draw_offsets()
     if n_rocks > 0:   # generate_state's draws, same order
         c = np.random.random((n_rocks, 2))
         c[:, 0] *= w * 0.75
@@ -177,7 +187,7 @@ def generate_episode(w, h, n_ants, n_pheromones, n_rocks, food_generator, walls_
     if draw_ant_seed:
         ep["seed"] = np.random.random(n_ants)
     ep["rw_prev_dist"] = _prev_dist(ep["x"], ep["y"], ep["anthill_xyr"])
-    if not (disc_inside(ep["wall_discs"], w, h) and disc_inside(ep["food_discs"], w, h)):
+    if not all(disc_inside(ep[k], w, h) for k in ("wall_discs", "food_discs") if k in ep):
         return None
     return ep
 
@@ -213,7 +223,7 @@ class BatchedEnvironmentGenerator:
             batch.activate_all_pheromones(np.ones((n_envs, self.n_ants, self.n_pheromones)) * 10.0)
         return batch
 
-    def reset(self, batch, seed_base, envs=None, float_activation=True):
+    def reset(self, batch, seed_base, envs=None, float_activation=True, perlin="host"):
         """A new episode for every env of `batch` (a BatchedAnts of this configuration), or with ``envs=(env0, n)`` for
         that window only (main.py:66-79 generates a new environment per episode).  Env e gets the episode drawn with
         seed ``seed_base + batch.env_id_base + e`` (its global id, as in `generate`), and the handle ends up in the state
@@ -222,7 +232,13 @@ class BatchedEnvironmentGenerator:
         With CirclesGenerator walls and food whose discs all lie inside the map, only the draws are made on the host
         (`generate_episode`) and the maps are written on the device (`BatchedAnts.generate_env_maps`); otherwise (Perlin
         walls, a duck-typed generator, a map smaller than a disc) the complete state is built on the host and imported.
-        Both give the same result.  -> "device" or "host", the path taken."""
+        With ``perlin="device"`` a layer of an exact `PerlinGenerator` takes the device path too: its two offsets are
+        drawn on the host and the noise is computed where the records are written, bit for bit as `perlin.py`.  The
+        default, ``perlin="host"``, keeps such maps on the host path; making "device" the default (and removing the
+        option) is meant to follow once its numbers are measured at scale.  Both paths give the same result.
+        -> "device" or "host", the path taken."""
+        if perlin not in ("host", "device"):
+            raise ValueError("perlin must be 'host' or 'device', not %r" % (perlin,))
         env0, n = (0, batch.E) if envs is None else (int(envs[0]), int(envs[1]))
         if env0 < 0 or n < 1 or env0 + n > batch.E:
             raise ValueError("env window (%d, %d) outside the batch of %d envs" % (env0, n, batch.E))
@@ -230,15 +246,20 @@ class BatchedEnvironmentGenerator:
         args = (self.w, self.h, self.n_ants, self.n_pheromones, self.n_rocks, self.food_generator, self.walls_generator)
         eps = []
         for s in seeds:
-            ep = generate_episode(*args, seed=s)
+            ep = generate_episode(*args, seed=s, perlin=perlin == "device")
             if ep is None:
                 break
             eps.append(ep)
         N, P = self.n_ants, self.n_pheromones
         if len(eps) == n:
             path = "device"
-            batch.generate_env_maps(np.stack([ep["anthill_xyr"] for ep in eps]), np.stack([ep["wall_discs"] for ep in eps]),
-                                    np.stack([ep["food_discs"] for ep in eps]), envs=(env0, n))
+            layers = []
+            for name, g in (("wall", self.walls_generator), ("food", self.food_generator)):
+                if name + "_perlin" in eps[0]:
+                    layers.append(g.layer(np.stack([ep[name + "_perlin"] for ep in eps])))
+                else:
+                    layers.append(np.stack([ep[name + "_discs"] for ep in eps]))
+            batch.generate_env_maps(np.stack([ep["anthill_xyr"] for ep in eps]), layers[0], layers[1], envs=(env0, n))
             keys = ("x", "y", "theta", "seed", "rw_prev_dist") + (("rock_centers", "rock_radii", "rock_weights")
                                                                   if self.n_rocks > 0 else ())
             st = {k: np.stack([ep[k] for ep in eps]) for k in keys}

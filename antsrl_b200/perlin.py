@@ -9,8 +9,12 @@ reference holds no test or golden vector for it, so this restatement of the pack
 12 + 4 edge gradients, single precision; `pnoise2` = the octave sum normalised by the amplitude sum) is
 **parity unpinned**: it is checked by known-answer properties of the algorithm (zero on the integer lattice,
 bounds, smoothness, period), not against outputs of the package.  It only shapes the walls bitmap, an input
-of the step loop; it runs on the host, once per episode, vectorised over the whole map.
+of the step loop; it runs on the host, once per episode, vectorised over the whole map.  The device computes the same
+float32 field bit for bit (antsrl_b200/csrc/ants_perlin.cuh): `perlin_noise_device`, and the Perlin layers of
+`BatchedAnts.generate_env_maps` that `BatchedEnvironmentGenerator.reset(..., perlin="device")` writes.
 """
+import collections
+import ctypes as C
 import random
 
 import numpy as np
@@ -98,6 +102,43 @@ def perlin_noise_generator(w, h, offset_x, offset_y, scale=22.0, octaves=2, pers
     return pnoise2(xs, ys, octaves=octaves, persistence=persistence, lacunarity=lacunarity, base=0).astype(np.float64)
 
 
+# A Perlin map layer in the form ants_generate_env_maps_ex takes (AntsPerlinLayer): offsets (n, 2) int32 of n envs, and
+# the generator's parameters, shared by the envs
+PerlinLayer = collections.namedtuple("PerlinLayer", "offsets scale density octaves persistence lacunarity")
+
+
+def perlin_layer_struct(layer):
+    """-> (AntsPerlinLayer, the contiguous int32 offsets it points to: keep it alive for the call)."""
+    from ._cabi import AntsPerlinLayer
+    offs = np.ascontiguousarray(layer.offsets, dtype=np.int32)
+    if offs.ndim != 2 or offs.shape[1] != 2:
+        raise ValueError("Perlin offsets must have shape (n, 2); got %r" % (offs.shape,))
+    s = AntsPerlinLayer()
+    s.offsets = offs.ctypes.data_as(C.POINTER(C.c_int32))
+    s.scale, s.density = float(layer.scale), float(layer.density)
+    s.octaves, s.reserved = int(layer.octaves), 0
+    s.persistence, s.lacunarity = float(layer.persistence), float(layer.lacunarity)
+    return s, offs
+
+
+def perlin_noise_device(w, h, offsets, scale=22.0, octaves=2, persistence=0.5, lacunarity=2.0, device=0):
+    """`perlin_noise_generator` on the GPU (ants_perlin_noise) for n offset pairs at once: offsets (n, 2) of
+    (offset_x, offset_y) -> float32 CUDA tensor (n, w, h), equal bit for bit to
+    ``perlin_noise_generator(w, h, ox, oy, ...).astype(np.float32)`` (the host function widens its float32 field to
+    float64).  The same device code writes the Perlin layers of `BatchedAnts.generate_env_maps`."""
+    import torch
+    from ._cabi import check, load_library
+    lib = load_library()
+    layer, offs = perlin_layer_struct(PerlinLayer(offsets, scale, 0.0, octaves, persistence, lacunarity))
+    dev = torch.device("cuda", device)
+    out = torch.empty((offs.shape[0], int(w), int(h)), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream().cuda_stream
+        check(lib, lib.ants_perlin_noise(int(device), C.byref(layer), offs.shape[0], int(w), int(h),
+                                         C.c_void_p(out.data_ptr()), C.c_void_p(stream)))
+    return out
+
+
 class PerlinGenerator:
     """map_generators.py:9-25: walls where the noise exceeds `density`; draws the two offsets from the global
     `random` module exactly like the reference (so the draws that follow it stay aligned)."""
@@ -106,9 +147,23 @@ class PerlinGenerator:
         self.scale, self.density, self.octaves = scale, density, octaves
         self.persistence, self.lacunarity = persistence, lacunarity
 
-    def generate(self, w, h):
+    def draw_offsets(self):
+        """-> int32 (offset_x, offset_y): exactly the two `random.randint` calls of `generate`, in its order."""
         offset_x = random.randint(-10000, 10000)
         offset_y = random.randint(-10000, 10000)
+        return np.array([offset_x, offset_y], dtype=np.int32)
+
+    def stamp(self, w, h, offsets):
+        """bool (w, h): the map of the drawn offsets, noise > density."""
+        offset_x, offset_y = (int(v) for v in offsets)
         return perlin_noise_generator(w, h, offset_x=offset_x, offset_y=offset_y, scale=self.scale,
                                       octaves=self.octaves, persistence=self.persistence,
                                       lacunarity=self.lacunarity) > self.density
+
+    def generate(self, w, h):
+        return self.stamp(w, h, self.draw_offsets())
+
+    def layer(self, offsets):
+        """The PerlinLayer of this generator for the (n, 2) offsets of n envs (BatchedAnts.generate_env_maps)."""
+        return PerlinLayer(np.asarray(offsets, dtype=np.int32).reshape(-1, 2), self.scale, self.density, self.octaves,
+                           self.persistence, self.lacunarity)

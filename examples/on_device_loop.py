@@ -6,11 +6,12 @@ observation -> epsilon-greedy action (a torch MLP with the collect agents' two h
 -> update, for E environments at once.  Observations, actions, rewards and the replay memory never cross PCIe; the
 only host traffic per step is kernel launches.  PyTorch is plumbing (the MLP and the ring-buffer copies).
 
-    python examples/on_device_loop.py [--envs 512] [--steps 50] [--workload cfg4] [--episodes K]
+    python examples/on_device_loop.py [--envs 512] [--steps 50] [--workload cfg4] [--episodes K] [--walls perlin]
 
 With --episodes K > 1 an episode lasts --steps steps, and when `done` arrives every env starts a new one
 (main.py:66-79) through BatchedEnvironmentGenerator.reset, which writes the new maps on the device; the share of the
-wall time spent in those resets is printed.
+wall time spent in those resets is printed.  With --walls perlin the walls are main.py's default PerlinGenerator()
+(main.py:75) instead of the workload's discs; its maps are written on the device too (reset(..., perlin="device")).
 """
 import argparse
 import os
@@ -25,7 +26,7 @@ import torch         # noqa: E402
 
 import bench         # noqa: E402
 from antsrl_b200 import BatchedAnts                      # noqa: E402
-from antsrl_b200.generator import stack_states           # noqa: E402
+from antsrl_b200.generator import PerlinGenerator, stack_states   # noqa: E402
 from antsrl_b200.replay import DeviceReplayMemory        # noqa: E402
 from antsrl_b200.device_loop import DeviceActionSelector  # noqa: E402
 
@@ -52,14 +53,21 @@ def main():
     ap.add_argument("--epsilon", type=float, default=0.3)
     ap.add_argument("--replay", type=int, default=1 << 20)
     ap.add_argument("--episodes", type=int, default=1, help="episodes of --steps steps each (1: one episode, no reset)")
+    ap.add_argument("--walls", choices=["circles", "perlin"], default="circles",
+                    help="the workload's CirclesGenerator walls, or main.py's default PerlinGenerator()")
     a = ap.parse_args()
     wl = bench.WORKLOADS[a.workload]
     E, N = a.envs, wl["n_ants"]
     gen = bench.make_generator(wl, a.steps + 10 if a.episodes <= 1 else a.steps)
-    states = bench.generate_states_parallel(wl, a.steps + 10, 0, E)
+    perlin = "device" if a.walls == "perlin" else "host"
     env = BatchedAnts(gen.cfg, E, evap_mode="lazy", record="compact8")
-    env.import_state(stack_states(states, "all"))
-    env.activate_all_pheromones(np.ones((E, N, wl["n_phero"])) * 10.0)          # agent.initialize
+    if a.walls == "perlin":
+        gen.walls_generator = PerlinGenerator()                                  # main.py:75
+        gen.reset(env, gen.seed_base, perlin=perlin)                             # = gen.generate(E), maps on the device
+    else:
+        states = bench.generate_states_parallel(wl, a.steps + 10, 0, E)
+        env.import_state(stack_states(states, "all"))
+        env.activate_all_pheromones(np.ones((E, N, wl["n_phero"])) * 10.0)      # agent.initialize
     C = len(gen.cfg["channels"])
     policy = TwoHeadPolicy(49 * C, 2).cuda().half()
     mem = DeviceReplayMemory(a.replay, (7, 7, C), (2,), 2)
@@ -86,7 +94,7 @@ def main():
         if done and a.episodes > 1 and episode + 1 < a.episodes:                # main.py:66-79: a new environment
             episode += 1
             r0 = time.perf_counter()
-            gen.reset(env, gen.seed_base + episode * E)                          # (reset synchronises the stream)
+            gen.reset(env, gen.seed_base + episode * E, perlin=perlin)           # (reset synchronises the stream)
             obs, ast, _, _ = env.observe()
             obs, ast = obs.clone(), ast.clone()
             torch.cuda.synchronize()

@@ -164,6 +164,38 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
 int ants_generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr, int32_t n_wall_discs,
                            const int32_t *wall_discs, int32_t n_food_discs, const int32_t *food_discs);
 
+/* A map layer of PerlinGenerator (map_generators.py:9-25, the reference's default walls): env e's layer is set at cell
+ * (x, y) iff (double)pnoise2(x', y', octaves, persistence, lacunarity, repeat 1024) > density, with
+ * x' = (float)((double)(x + offset_x) / scale) and y' likewise (utils.perlin_noise_generator; the float32 algorithm of
+ * antsrl_b200/perlin.py, bit for bit).  The generator's parameters are shared by the envs; the offsets are the two
+ * random.randint(-10000, 10000) draws of each env. */
+typedef struct AntsPerlinLayer {
+    const int32_t *offsets;      /* host [n_envs][2]: (offset_x, offset_y) of each env */
+    double scale;                /* x = (float)((double)(cell_x + offset_x) / scale), y likewise */
+    double density;              /* a cell is set iff (double)pnoise2(x, y) > density */
+    int32_t octaves;             /* 1 ... 32 */
+    int32_t reserved;
+    double persistence, lacunarity;   /* rounded to float, as pnoise2 does */
+} AntsPerlinLayer;
+/* ants_generate_env_maps with layers that may be Perlin noise: a layer whose *_perlin pointer is non-NULL is that noise
+ * (its disc count must be 0), otherwise it is the discs, exactly as ants_generate_env_maps.  Walls and food follow the
+ * same rules (a wall outside the anthill disc; food 1.0 where the food layer is set and the cell is not a wall).
+ * ANTS_E_ARG, with the handle unchanged, for what ants_generate_env_maps rejects and for: octaves outside 1 ... 32; a
+ * scale that is 0 or not finite; a persistence or lacunarity that is not finite; a layer given both discs and Perlin
+ * noise; NULL offsets; an octave whose period 1024 * freq (in float) is 0, not finite or at least 2^31 in magnitude; a
+ * map edge whose coordinate x' * freq (in float) is not finite or at least 2^31 in magnitude (the integer parts of the
+ * noise stay in int32). */
+int ants_generate_env_maps_ex(AntsBatch *b, int32_t env0, int32_t n_envs, const int32_t *anthill_xyr,
+                              int32_t n_wall_discs, const int32_t *wall_discs, const AntsPerlinLayer *wall_perlin,
+                              int32_t n_food_discs, const int32_t *food_discs, const AntsPerlinLayer *food_perlin);
+/* utils.perlin_noise_generator on the device, without a handle: the float32 field pnoise2 (the value before the density
+ * threshold, which is ignored) of the n offset pairs of `layer` on a w x h map, written to the DEVICE buffer
+ * d_out [n][w][h] on `stream` (a cudaStream_t, NULL = the legacy default stream) of CUDA device `device`; returns when
+ * the field is written.  The same device code as the Perlin layers of ants_generate_env_maps_ex, and the same
+ * ANTS_E_ARG cases. */
+int ants_perlin_noise(int32_t device, const AntsPerlinLayer *layer, int32_t n, int32_t w, int32_t h, float *d_out,
+                      void *stream);
+
 /* Ants.activate_all_pheromones, ants.py:86-87.  act: host [E][N][P] */
 int ants_activate_all_pheromones(AntsBatch *b, const double *act, int32_t is_bool);
 

@@ -12,7 +12,13 @@
 Both resets are made from the same seeds and their states compared (two envs, every key).  Prints one JSON line per
 workload; the GPU name and power limit are read in the same run.
 
-    python scripts/reset_bench.py [--workloads cfg4 cfg3] [--launches 25]
+With --walls perlin the workload's walls are the reference's default PerlinGenerator() (main.py:75) instead, and the
+script reports reset(perlin="host") end to end (host noise over every cell, complete import), the host draws
+(generate_episode(perlin=True)), the generate_env_maps call, the Perlin kernel's CUDA-event median next to the Circles
+kernel's median on the same window in the same run (the yardstick of the Perlin kernel), the memset yardstick, the
+per-ant import, reset(perlin="device") end to end, and a two-env comparison of the two paths.
+
+    python scripts/reset_bench.py [--workloads cfg4 cfg3] [--launches 25] [--walls {circles,perlin}]
 """
 import argparse
 import json
@@ -173,17 +179,111 @@ def run(name, launches):
     return res
 
 
+def _kernel_median(b, launches, hill, walls, food):
+    """generate_env_maps on the whole batch: the call's wall time and the `reset` family's CUDA-event time, medians over
+    `launches` calls after 3 warm-up calls."""
+    for _ in range(3):
+        b.generate_env_maps(hill, walls, food)
+    b.set_profiling(True)
+    call_s, kern_ms = [], []
+    for _ in range(launches):
+        b.reset_kernel_ms()
+        dt, _ = wall(lambda: b.generate_env_maps(hill, walls, food))
+        call_s.append(dt)
+        ms, n = b.kernel_ms()["reset"]
+        assert n == 1
+        kern_ms.append(ms)
+    b.set_profiling(False)
+    return statistics.median(call_s), statistics.median(kern_ms), [min(kern_ms), max(kern_ms)]
+
+
+def run_perlin(name, launches):
+    import torch
+    from antsrl_b200 import BatchedAnts
+    from antsrl_b200.generator import PerlinGenerator, generate_episode
+    wl = bench.WORKLOADS[name]
+    E, N, W, H, P = wl["envs_per_gpu"], wl["n_ants"], wl["w"], wl["h"], wl["n_phero"]
+    circles = bench.make_generator(wl, 1000)
+    gen = bench.make_generator(wl, 1000)
+    gen.walls_generator = PerlinGenerator()
+    b = BatchedAnts(gen.cfg, E, evap_mode="lazy", record="compact8")
+    res = {"workload": name, "walls": "PerlinGenerator()", "envs": E, "map": [W, H], "ants_per_env": N,
+           "record": "compact8"}
+    g = gen
+    res["draws_one_process_s"], eps = wall(lambda: [generate_episode(g.w, g.h, N, P, g.n_rocks, g.food_generator,
+                                                                     g.walls_generator, seed=g.seed_base + e,
+                                                                     perlin=True) for e in range(E)])
+    hill = np.stack([e["anthill_xyr"] for e in eps])
+    layer, fd = g.walls_generator.layer(np.stack([e["wall_perlin"] for e in eps])), np.stack([e["food_discs"] for e in eps])
+    res["generate_env_maps_call_s_median"], res["perlin_kernel_ms_median"], res["perlin_kernel_ms_min_max"] = \
+        _kernel_median(b, launches, hill, layer, fd)
+    c_eps = [generate_episode(W, H, N, P, circles.n_rocks, circles.food_generator, circles.walls_generator,
+                              seed=circles.seed_base + e) for e in range(E)]
+    _, res["circles_kernel_ms_median"], res["circles_kernel_ms_min_max"] = _kernel_median(
+        b, launches, np.stack([e["anthill_xyr"] for e in c_eps]), np.stack([e["wall_discs"] for e in c_eps]),
+        np.stack([e["food_discs"] for e in c_eps]))
+    res["kernel_launches_timed"] = launches
+    res["perlin_over_circles_kernel"] = res["perlin_kernel_ms_median"] / res["circles_kernel_ms_median"]
+    res["perlin_kernel_within_2x_of_circles"] = bool(res["perlin_over_circles_kernel"] <= 2.0)
+    written = E * (-(-W // 16) * 16) * (-(-H // 16) * 16) * 8
+    res["kernel_bytes_written"] = written
+    buf = torch.empty(written, dtype=torch.uint8, device="cuda")
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
+    ms_set = []
+    for k in range(13):
+        ev[0].record()
+        buf.zero_()
+        ev[1].record()
+        torch.cuda.synchronize()
+        if k >= 3:
+            ms_set.append(ev[0].elapsed_time(ev[1]))
+    del buf
+    res["memset_same_bytes_ms_median"] = statistics.median(ms_set)
+    ants = {k: np.stack([e[k] for e in eps]) for k in ("x", "y", "theta", "seed", "rw_prev_dist")}
+    if g.n_rocks:
+        ants.update({k: np.stack([e[k] for e in eps]) for k in ("rock_centers", "rock_radii", "rock_weights")})
+    ants.update(prev_x=ants["x"], prev_y=ants["y"], prev_theta=ants["theta"], holding=np.zeros((E, N)),
+                rewards=np.zeros((E, N)), rw_holding_prev=np.zeros((E, N)), mandibles=np.zeros((E, N), np.uint8),
+                reward_state=np.zeros((E, N), np.uint8), anthill_food=np.zeros(E),
+                activation=np.full((E, N, P), 10.0), timestep=1, rw_alias=True, act_bool=False)
+    t_ant = []
+    for _ in range(5):
+        dt, _ = wall(lambda: b.import_state(ants))
+        t_ant.append(dt)
+    res["per_ant_import_s_median"] = statistics.median(t_ant)
+    t_reset = []
+    for _ in range(3):
+        dt, path = wall(lambda: (gen.reset(b, gen.seed_base, perlin="device"), b.synchronize())[0])
+        assert path == "device"
+        t_reset.append(dt)
+    res["device_reset_one_process_s_median"] = statistics.median(t_reset)
+    dev_state = b.export_state(envs=(0, 2))
+    dt_host, path = wall(lambda: (gen.reset(b, gen.seed_base), b.synchronize())[0])
+    assert path == "host"
+    res["host_reset_one_process_s"] = dt_host
+    host_state = b.export_state(envs=(0, 2))
+    res["device_reset_equals_host_reset"] = bool(all(
+        np.array_equal(v, host_state[k]) if isinstance(v, np.ndarray) else v == host_state[k]
+        for k, v in dev_state.items()))
+    res["speedup_reset_call"] = dt_host / res["device_reset_one_process_s_median"]
+    b.close()
+    torch.cuda.synchronize()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--workloads", nargs="+", default=["cfg4", "cfg3"], choices=sorted(bench.WORKLOADS))
     ap.add_argument("--launches", type=int, default=25, help="timed k_reset_maps launches (median)")
+    ap.add_argument("--walls", choices=["circles", "perlin"], default="circles",
+                    help="the workload's CirclesGenerator walls, or the reference's default PerlinGenerator()")
     a = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("reset_bench.py measures on a CUDA device; there is none")
     info = gpu_info()
     for name in a.workloads:
-        r = run(name, max(a.launches, 20))
+        r = (run if a.walls == "circles" else run_perlin)(name, max(a.launches, 20))
         r.update(info)
         print(json.dumps(r), flush=True)
 
