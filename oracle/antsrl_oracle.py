@@ -160,8 +160,8 @@ class OracleEnv:
         self.filter = diffuse_filter(cfg["diffuse_factor"], cfg["evap_factor"])
 
     # ------------------------------------------------------------------ observation (RL_api.py:96-165)
-    def sample_cells(self):
-        """Integer sample coordinates (N,S,S,2) of every ant, RL_api.py:100-119."""
+    def sample_points(self):
+        """Sample coordinates (N,S,S,2) of every ant before rounding, RL_api.py:100-116."""
         s, cfg = self.s, self.cfg
         xy = np.stack([s["x"], s["y"]], axis=1)
         theta = s["theta"]
@@ -175,8 +175,12 @@ class OracleEnv:
         rx = cos_t[:, AX, AX] * rel[:, :, :, 0] - sin_t[:, AX, AX] * rel[:, :, :, 1]
         ry = sin_t[:, AX, AX] * rel[:, :, :, 0] + cos_t[:, AX, AX] * rel[:, :, :, 1]
         rel[:, :, :, 0], rel[:, :, :, 1] = rx, ry
-        ab = rel + xy_f[:, AX, AX, :]
-        ab = np.round(ab).astype(int)                    # half-to-even, Q11
+        return rel + xy_f[:, AX, AX, :]
+
+    def sample_cells(self):
+        """Integer sample coordinates (N,S,S,2) of every ant, RL_api.py:100-119."""
+        cfg = self.cfg
+        ab = np.round(self.sample_points()).astype(int)  # half-to-even, Q11
         ab[:, :, :, 0] = np.mod(ab[:, :, :, 0], cfg["w"])
         ab[:, :, :, 1] = np.mod(ab[:, :, :, 1], cfg["h"])
         return ab
