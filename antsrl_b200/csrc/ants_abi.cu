@@ -177,6 +177,8 @@ struct AntsBatch {
     int rw_alias = 1, act_bool = 1, prev_synced = 1, needs_sweep = 1;
     int wall_flags_valid = 0;       // wall_hit[] was written by the step that precedes this update
     int absorb_par = 0;             // which absorb counter the steps append under
+    int steps_queued = 0;           // flat kernels: steps since the last update (each may queue up to E * N absorbs; the
+                                    // list holds E * N, so a second one makes the update sweep every disc instead)
     int commit_par = 0;             // which commit counter this step appends under
     int use_pdl = 0;                // programmatic dependent launch of the step kernels (large batches)
     CUtensorMap plane_map;          // diffusion mode: {H, W, 2 * E * P} f64 over both pheromone planes, box 68 x 66 x 1
@@ -687,6 +689,7 @@ int do_step(AntsBatch *b, const int8_t *d_rot, const int8_t *d_ph, float *d_obs,
         b->commit_par ^= 1;
     }
     TRY(check_launch("k_food_commit"));
+    if (++b->steps_queued > 1) b->needs_sweep = 1;   // the absorb list may have overflowed (k_food_commit)
     b->prev_synced = 0;
     b->wall_flags_valid = 1;
     TRY(launch_perceive(b, d_obs, d_as, nullptr, d_reward, 1));
@@ -774,13 +777,15 @@ int do_update(AntsBatch *b, const double *d_noise) {
         TRY(check_launch("k_deposit_commit"));
     }
     // 7. Anthill (order 1000): the queued cells were absorbed by the first blocks of k_collide; after an import one
-    //    sweep over the disc takes whatever the generator put there (Q10)
+    //    sweep over the disc takes whatever the generator put there (Q10), after several steps without an update
+    //    whatever did not fit the list
     if (b->needs_sweep) {
         LaunchScope ls(b, F_ABSORB);
         ants::k_absorb_sweep<<<p.E, 256, 0, b->stream>>>(p);
         b->needs_sweep = 0;
         TRY(check_launch("absorb"));
     }
+    b->steps_queued = 0;
     b->prev_synced = 1;
     b->stats.updates++;
     return ANTS_OK;
@@ -1379,13 +1384,13 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     if (p.owner) CK(cudaMemsetAsync(p.owner, 0, (size_t)p.E * p.plane * sizeof(uint32_t), st));
     b->move_done = 0;
     if (s->food) b->pack_disabled = 0;
-    // queued anthill absorbs refer to the old food field / disc: dropped only when one of them is replaced (the
-    // sweep of the next update takes whatever lies in the disc, Q10)
+    // queued anthill absorbs refer to the old food field / disc: dropped when one of them is replaced (the sweep of the
+    // next update takes whatever lies in the disc, Q10).  The flat kernels keep one batch-wide queue, so a partial import
+    // drops all of it: an entry of a replaced env may name a cell outside its new disc, and the entries of the other envs
+    // lie in discs that the same sweep covers.
     if (s->food || s->anthill_xyr) {
         if (b->fused) CK(cudaMemsetAsync(p.absorb_count + env0, 0, (size_t)n_envs * sizeof(uint32_t), st));
-        else if (whole) CK(cudaMemsetAsync(p.absorb_count, 0, 2 * sizeof(uint32_t), st));
-        // (flat kernels, partial import: the batch-wide queue is kept; its cells are absorbed by the next update, which
-        //  is what the sweep of that update would do to them anyway)
+        else CK(cudaMemsetAsync(p.absorb_count, 0, 2 * sizeof(uint32_t), st));
     }
     if (s->x || s->y) b->wall_flags_valid = 0;
     b->owner_phase = 0;
@@ -1539,7 +1544,7 @@ static int generate_env_maps(AntsBatch *b, int32_t env0, int32_t n_envs, const i
     // the same bookkeeping as an import of food, walls, explored, pheromones and the anthill (ants_import_env_state)
     if (p.owner) CK(cudaMemsetAsync(p.owner, 0, (size_t)p.E * p.plane * sizeof(uint32_t), st));
     if (b->fused) CK(cudaMemsetAsync(p.absorb_count + env0, 0, (size_t)n_envs * sizeof(uint32_t), st));
-    else if (whole) CK(cudaMemsetAsync(p.absorb_count, 0, 2 * sizeof(uint32_t), st));
+    else CK(cudaMemsetAsync(p.absorb_count, 0, 2 * sizeof(uint32_t), st));   // (the whole batch-wide queue, as above)
     b->needs_sweep = 1;                                     // food may lie inside the new anthill disc (Q10)
     b->move_done = 0;
     b->pack_disabled = 0;

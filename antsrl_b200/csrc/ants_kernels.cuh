@@ -529,9 +529,12 @@ __global__ void __launch_bounds__(128) k_food_commit(Params p, uint32_t owner_st
         st_food(p, fr, nv);
         nv = ld_food(p, fr);                                                   // as stored (f32 in compact records)
         if (nv != 0.0 && in_hill(p.hill + 4 * e, pcx, pcy)) {
+            // (the list holds E * N pairs, one step's worth: past that the update sweeps every disc instead)
             uint32_t s = atomicAdd(p.absorb_count + par, 1u);
-            p.absorb_list[2 * s] = (uint32_t)e;
-            p.absorb_list[2 * s + 1] = (uint32_t)pcell;
+            if (s < (uint32_t)p.EN) {
+                p.absorb_list[2 * s] = (uint32_t)e;
+                p.absorb_list[2 * s + 1] = (uint32_t)pcell;
+            }
         }
     }
 }
@@ -886,9 +889,10 @@ k_collide(Params p, const double *__restrict__ noise, uint32_t step_id, uint32_t
           int par) {
     pdl_begin();
     // Anthill.update (anthill.py:41-46) for the cells queued by k_food_commit: nothing else in the update reads the
-    // food field, so the first blocks of this kernel absorb them; the other counter is zeroed for the next step.
+    // food field, so the first blocks of this kernel absorb them; the other counter is zeroed for the next step.  (A
+    // count past E * N means the list overflowed: the update then sweeps every disc, k_absorb_sweep.)
     {
-        const uint32_t n = p.absorb_count[par];
+        const uint32_t n = min(p.absorb_count[par], (uint32_t)p.EN);
         const uint32_t nb = gridDim.x < 32u ? gridDim.x : 32u;
         if (blockIdx.x < nb) {
             for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += nb * blockDim.x) {
