@@ -1287,6 +1287,13 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     Params &p = b->p;
     if (env0 < 0 || n_envs < 1 || (int64_t)env0 + n_envs > p.E)
         return fail(ANTS_E_ARG, "env window [%d, %d) outside the batch of %d envs", env0, env0 + n_envs, p.E);
+    if (p.diffuse && s->activation) {                  // a plane value's sign bit is the wall flag: no negative deposits
+        const size_t n = (size_t)n_envs * p.N * p.P;
+        for (size_t i = 0; i < n; ++i)
+            if (!(s->activation[i] >= 0.0))
+                return fail(ANTS_E_ARG, "env %d, ant %d: activation %g; with diffusion an activation must be >= 0",
+                            env0 + (int)(i / ((size_t)p.N * p.P)), (int)(i / p.P % p.N), s->activation[i]);
+    }
     CK(cudaSetDevice(b->cfg.device));
     cudaStream_t st = b->stream;
     const bool whole = n_envs == p.E;
@@ -1320,8 +1327,11 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     // map fields: dense host array -> device scratch -> pack kernel into the cell records
     const size_t ncell = (size_t)n_envs * p.W * p.H;
     Scratch scratch;
+    size_t scratch_flag_off = 0;                                           // one word after the data: k_plane_walls's flag
     if (s->phero || s->food || s->walls || s->explored) {
         size_t need = ncell * 8 * ((s->phero && p.P > 1) ? p.P : 1);
+        scratch_flag_off = need;
+        need += sizeof(uint32_t);
         cudaError_t me = cudaMalloc(&scratch.ptr, need);
         if (me != cudaSuccess) return fail(ANTS_E_ALLOC, "import scratch of %zu bytes: %s", need, cudaGetErrorString(me));
     }
@@ -1347,9 +1357,13 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
         ants::k_pack_u8<<<148 * 8, 256, 0, st>>>(p, (const uint8_t *)d_tmp, 0, env0, n_envs);      // Walls.__init__: astype(bool)
         TRY(check_launch("k_pack_u8"));
     }
+    uint32_t bad_phero = 0;
     if (p.diffuse && (s->walls || s->phero)) {         // the planes carry the wall bit in their sign
-        ants::k_plane_walls<<<148 * 8, 256, 0, st>>>(p, env0, n_envs);
+        uint32_t *d_bad = s->phero ? (uint32_t *)((char *)d_tmp + scratch_flag_off) : nullptr;
+        if (d_bad) CK(cudaMemsetAsync(d_bad, 0, sizeof(uint32_t), st));
+        ants::k_plane_walls<<<148 * 8, 256, 0, st>>>(p, env0, n_envs, d_bad);
         TRY(check_launch("k_plane_walls"));
+        if (d_bad) CK(cudaMemcpyAsync(&bad_phero, d_bad, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     }
     if (s->explored) {
         CK(cudaMemcpyAsync(d_tmp, s->explored, ncell, cudaMemcpyHostToDevice, st));
@@ -1399,6 +1413,9 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     if (s->rw_alias >= 0) b->rw_alias = s->rw_alias ? 1 : 0;
     if (s->act_bool >= 0) b->act_bool = s->act_bool ? 1 : 0;
     CK(cudaStreamSynchronize(st));   // host temporaries above must outlive the copies
+    if (bad_phero)
+        return fail(ANTS_E_ARG, "an imported pheromone value is negative or NaN; with diffusion values must be >= 0 "
+                    "(import the window again)");
     return ANTS_OK;
 }
 
@@ -1685,6 +1702,9 @@ int ants_activate_all_pheromones(AntsBatch *b, const double *act, int32_t is_boo
     for (int64_t i = 0; i < p.EN; ++i)
         for (int k = 0; k < p.P; ++k) {
             double v = act[i * p.P + k];
+            if (p.diffuse && !is_bool && !(v >= 0.0))  // a plane value's sign bit is the wall flag: no negative deposits
+                return fail(ANTS_E_ARG, "env %d, ant %d: activation %g; with diffusion an activation must be >= 0",
+                            (int)(i / p.N), (int)(i % p.N), v);
             act_t[(size_t)k * p.EN + i] = is_bool ? (v != 0.0 ? 1.0 : 0.0) : v;
         }
     CK(cudaMemcpyAsync(p.act, act_t.data(), act_t.size() * sizeof(double), cudaMemcpyHostToDevice, b->stream));

@@ -1227,8 +1227,10 @@ k_diffuse_tma(Params p, const __grid_constant__ CUtensorMap tmap, int src_z0, in
         }
     }
 }
-// after an import: the sign bit of every plane value = the wall bit of its cell record
-__global__ void k_plane_walls(Params p, int env0, int n_env) {
+// after an import: the sign bit of every plane value = the wall bit of its cell record.  `bad` (non-null when the
+// planes were just imported, so they still hold the caller's values): set to 1 if one of them is negative or NaN --
+// the sign bit is the wall flag, so such a value cannot be represented (ants_import_env_state rejects the import)
+__global__ void k_plane_walls(Params p, int env0, int n_env, uint32_t *bad) {
     const int64_t n = (int64_t)n_env * p.W * p.H;
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
         int64_t ex = j / p.H;
@@ -1239,7 +1241,8 @@ __global__ void k_plane_walls(Params p, int env0, int n_env) {
         const bool wall = ld_wall(p, rec_at(p, (int)e, cidx(p, x, y)));
         for (int k = 0; k < p.P; ++k) {
             double *pv = plane_at(p, (int)e, k, x, y);
-            const double a = fabs(*pv);
+            const double v = *pv, a = fabs(v);
+            if (bad != nullptr && !(v >= 0.0)) *bad = 1u;
             *pv = wall ? -a : a;
         }
     }

@@ -152,6 +152,10 @@ int ants_export_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, AntsHostSt
 /* ... and the import of such a window: a new map / new ants for the envs [env0, env0 + n_envs) only (main.py:66-79
  * generates a new environment per episode), or a large batch uploaded in slices.  The scalars stay batch-wide. */
 int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const AntsHostState *s);
+/* With DIFFUSE_FACTOR != 0 the sign bit of a pheromone plane value is the wall flag of its cell, so negative and NaN
+ * pheromone values cannot be represented there (the reference allows them): ants_import_env_state returns ANTS_E_ARG
+ * for such an activation before it uploads anything, and for such a pheromone value after the window's import has
+ * run -- the window must then be imported again. */
 /* A new episode's map for the envs [env0, env0 + n_envs), written on the device from the generator's random draws
  * instead of dense planes (EnvironmentGenerator.generate, environment_generator.py:60-72, with CirclesGenerator walls
  * and food).  Host arrays: anthill_xyr [n_envs][3], wall_discs [n_envs][n_wall_discs][3], food_discs
@@ -196,7 +200,8 @@ int ants_generate_env_maps_ex(AntsBatch *b, int32_t env0, int32_t n_envs, const 
 int ants_perlin_noise(int32_t device, const AntsPerlinLayer *layer, int32_t n, int32_t w, int32_t h, float *d_out,
                       void *stream);
 
-/* Ants.activate_all_pheromones, ants.py:86-87.  act: host [E][N][P] */
+/* Ants.activate_all_pheromones, ants.py:86-87.  act: host [E][N][P].  With DIFFUSE_FACTOR != 0, ANTS_E_ARG with the
+ * handle unchanged for a negative or NaN activation (the plane's sign bit is the wall flag). */
 int ants_activate_all_pheromones(AntsBatch *b, const double *act, int32_t is_bool);
 
 /* RLApi.observation(), RL_api.py:96-165 (side effect on reward state, as the reference).
