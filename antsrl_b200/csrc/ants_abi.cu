@@ -201,7 +201,7 @@ struct AntsBatch {
     int perceive_smem = 0, perceive_layout = 0, perceive_group = 4, perceive_threads = 128, perceive_slow_wrap = 0;
     int perceive_rows = 0, rows_smem = 0;   // 1 = k_perceive_rows serves this configuration (default channel list, 7x7 window)
     // block-per-environment kernels (ants_env_fused.cuh): move / update / update+move in one launch each
-    int fused = 0, env_group = 1, env_apt = 4, env_smem = 0, env_tpb = 256;
+    int fused = 0, env_group = 1, env_cap = 256, env_smem = 0;   // env_cap: ants per block (256, 512 or 1024)
     int move_done = 0;              // ants_rollout: the move of the coming step already ran inside the last update launch
     // packed observation transport of the host-buffer path (ants_pack.cuh)
     AntsPackedLayout pack_layout;
@@ -221,9 +221,8 @@ struct AntsBatch {
     struct Group { cudaStream_t s = nullptr; cudaEvent_t done = nullptr; int env0 = 0, env1 = 0; };
     std::vector<Group> groups;
     cudaEvent_t ev_fork = nullptr;
-    int grouped = 0;                // inside a grouped rollout (whole-batch passes must join the groups first)
-    cudaStream_t cur_stream = nullptr;   // target of the step-kernel launches: nullptr = the handle's stream, whole batch
-    int cur_env0 = 0, cur_env1 = 0;
+    int grouped = 0;                // inside a grouped rollout: the step kernels launch once per group, whole-batch
+                                    // passes join the groups first
     // ants_generate_env_maps: device copy of the window's discs (grows to the largest window seen, freed by ants_destroy)
     int4 *reset_discs = nullptr;
     int64_t reset_cap = 0;
@@ -317,13 +316,14 @@ struct Scratch {                   // device scratch of import / export, freed o
 // touches memory.  Off while profiling (events between the launches), with ANTS_NO_PDL set, and for small batches
 // (measured: +1.5 % at 524 288 ants per launch, but the attribute's host cost loses 18 % at 51 200).
 template <typename... KArgs, typename... Args>
-void launch_step(AntsBatch *b, void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem, Args... args) {
+void launch_step(AntsBatch *b, cudaStream_t stream, void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem,
+                 Args... args) {
     static const bool env_off = getenv("ANTS_NO_PDL") != nullptr;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(block);
     cfg.dynamicSmemBytes = smem;
-    cfg.stream = b->cur_stream ? b->cur_stream : b->stream;
+    cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -339,7 +339,7 @@ int check_launch(const char *what) {
 }
 
 // grouped rollout: the groups' streams branch off the handle's stream and join it again; a whole-batch pass in between
-// (generation fold, lazy-field fold) joins them first
+// (generation fold, lazy-field fold, anthill sweep) joins them first
 void fork_groups(AntsBatch *b) {
     cudaEventRecord(b->ev_fork, b->stream);
     for (auto &g : b->groups) cudaStreamWaitEvent(g.s, b->ev_fork, 0);
@@ -395,33 +395,26 @@ uint32_t next_owner_phase(AntsBatch *b) {
     return ++b->owner_phase;
 }
 
-int launch_perceive_range(AntsBatch *b, uint32_t og, float *d_obs, float *d_as, float *d_state, double *d_reward, int is_step);
-
+// The perception kernel.  In a grouped rollout the row kernel launches once per group of environments on the group's
+// stream; otherwise (and always for the generic kernel, which has no env range) once over the whole batch.
 int launch_perceive(AntsBatch *b, float *d_obs, float *d_as, float *d_state, double *d_reward, int is_step) {
-    const uint32_t og = next_obs_gen(b);
-    TRY(launch_perceive_range(b, og, d_obs, d_as, d_state, d_reward, is_step));
-    b->rw_alias = 0;
-    return ANTS_OK;
-}
-
-// the perception kernel over the current launch target (whole batch, or one group of a grouped rollout)
-int launch_perceive_range(AntsBatch *b, uint32_t og, float *d_obs, float *d_as, float *d_state, double *d_reward, int is_step) {
     const Params &p = b->p;
-    const int64_t ant0 = b->cur_stream ? (int64_t)b->cur_env0 * p.N : 0, ant1 = b->cur_stream ? (int64_t)b->cur_env1 * p.N : p.EN;
-    int blocks = 0;
-    {
-        LaunchScope ls(b, F_PERCEIVE);
-        // (the straight-line layouts of k_perceive decode pheromones from the record words; in diffusion mode the field
-        //  lives in the f64 planes, which only its generic channel code reads)
-        const int layout = (p.diffuse && !b->perceive_rows) ? 0 : b->perceive_layout;
-        const uint32_t magic = (1u << 20) / (uint32_t)p.S2 + 1u;   // f / S2 == (f * magic) >> 20 for f < 2048
-        const int threads = b->perceive_threads;
-        blocks = (int)cdiv(p.EN, threads);
-        if (b->perceive_rows) {
+    const uint32_t og = next_obs_gen(b);
+    // (the straight-line layouts of k_perceive decode pheromones from the record words; in diffusion mode the field
+    //  lives in the f64 planes, which only its generic channel code reads)
+    const int layout = (p.diffuse && !b->perceive_rows) ? 0 : b->perceive_layout;
+    if (b->perceive_rows) {
+        const AntsBatch::Group whole = {b->stream, nullptr, 0, p.E};
+        const AntsBatch::Group *gs = b->grouped ? b->groups.data() : &whole;
+        const int n = b->grouped ? (int)b->groups.size() : 1;
+        for (int k = 0; k < n; ++k) {
+            const int64_t ant0 = (int64_t)gs[k].env0 * p.N, ant1 = (int64_t)gs[k].env1 * p.N;
             const int rblocks = (int)cdiv(ant1 - ant0, ants::kRowsThreads);
-#define ANTS_ROWS(L, R16, SS)                                                                               \
-    launch_step(b, ants::k_perceive_rows<L, R16, SS>, (unsigned)rblocks, (unsigned)ants::kRowsThreads,      \
-                (size_t)b->rows_smem, p, d_obs, d_as, d_state, d_reward, og, b->occ_gen, is_step,          \
+            {
+                LaunchScope ls(b, F_PERCEIVE);
+#define ANTS_ROWS(L, R16, SS)                                                                                     \
+    launch_step(b, gs[k].s, ants::k_perceive_rows<L, R16, SS>, (unsigned)rblocks, (unsigned)ants::kRowsThreads,   \
+                (size_t)b->rows_smem, p, d_obs, d_as, d_state, d_reward, og, b->occ_gen, is_step,                \
                 b->rw_alias, b->lazy_now, b->lazy_abs, ant0, ant1)
 #define ANTS_ROWS_S(SS)                                                                          \
     do {                                                                                         \
@@ -429,44 +422,88 @@ int launch_perceive_range(AntsBatch *b, uint32_t og, float *d_obs, float *d_as, 
         else if (p.rec16) { if (layout == 2) ANTS_ROWS(2, 1, SS); else ANTS_ROWS(1, 1, SS); }   \
         else { if (layout == 2) ANTS_ROWS(2, 0, SS); else ANTS_ROWS(1, 0, SS); }                \
     } while (0)
-            if (p.S == 7) ANTS_ROWS_S(7); else ANTS_ROWS_S(5);
+                if (p.S == 7) ANTS_ROWS_S(7); else ANTS_ROWS_S(5);
 #undef ANTS_ROWS_S
 #undef ANTS_ROWS
-        } else
-#define ANTS_PERCEIVE(L, R16)                                                                              \
-    launch_step(b, ants::k_perceive<L, R16>, (unsigned)blocks, (unsigned)threads, (size_t)b->perceive_smem, \
-                p, d_obs, d_as, d_state, d_reward, og, b->occ_gen, is_step, b->rw_alias, b->perceive_group, \
-                magic, b->perceive_slow_wrap, b->lazy_now, b->lazy_abs)
-        if (p.rec8) {                  // served through the generic channel code (accessor-based decode)
-            ANTS_PERCEIVE(0, false);
-        } else if (p.rec16) {
-            if (layout == 1) ANTS_PERCEIVE(1, true);
-            else if (layout == 2) ANTS_PERCEIVE(2, true);
-            else ANTS_PERCEIVE(0, true);
-        } else {
-            if (layout == 1) ANTS_PERCEIVE(1, false);
-            else if (layout == 2) ANTS_PERCEIVE(2, false);
-            else ANTS_PERCEIVE(0, false);
+            }
+            TRY(check_launch("k_perceive"));
         }
+    } else {
+        const uint32_t magic = (1u << 20) / (uint32_t)p.S2 + 1u;   // f / S2 == (f * magic) >> 20 for f < 2048
+        const int threads = b->perceive_threads;
+        const int blocks = (int)cdiv(p.EN, threads);
+        {
+            LaunchScope ls(b, F_PERCEIVE);
+#define ANTS_PERCEIVE(L, R16)                                                                                          \
+    launch_step(b, b->stream, ants::k_perceive<L, R16>, (unsigned)blocks, (unsigned)threads, (size_t)b->perceive_smem, \
+                p, d_obs, d_as, d_state, d_reward, og, b->occ_gen, is_step, b->rw_alias, b->perceive_group,             \
+                magic, b->perceive_slow_wrap, b->lazy_now, b->lazy_abs)
+            if (p.rec8) {                  // served through the generic channel code (accessor-based decode)
+                ANTS_PERCEIVE(0, false);
+            } else if (p.rec16) {
+                if (layout == 1) ANTS_PERCEIVE(1, true);
+                else if (layout == 2) ANTS_PERCEIVE(2, true);
+                else ANTS_PERCEIVE(0, true);
+            } else {
+                if (layout == 1) ANTS_PERCEIVE(1, false);
+                else if (layout == 2) ANTS_PERCEIVE(2, false);
+                else ANTS_PERCEIVE(0, false);
+            }
 #undef ANTS_PERCEIVE
+        }
+        TRY(check_launch("k_perceive"));
     }
-    return check_launch("k_perceive");
+    b->rw_alias = 0;
+    return ANTS_OK;
 }
 
 
 // ------------------------------------------------------------------------------------------------ block-per-env path
+// The block-per-environment kernel, once per group of environments on the group's stream in a grouped rollout, else
+// once over the whole batch.  Block shape from the ants per block: one ant per thread up to 512, 512 threads x 2 ants
+// for 1024 (ants_env_fused.cuh).
 template <bool UPDATE, bool MOVE>
-void launch_env(AntsBatch *b, ants::EnvArgs a) {
+int launch_env(AntsBatch *b, ants::EnvArgs a) {
+    constexpr int fam = UPDATE ? (MOVE ? F_ENV_FUSED : F_ENV_UPDATE) : F_ENV_MOVE;
+    const char *what = UPDATE ? (MOVE ? "k_env<update, move>" : "k_env<update>") : "k_env<move>";
     const Params &p = b->p;
-    a.env_base = b->cur_stream ? b->cur_env0 : 0;
-    a.env_end = b->cur_stream ? b->cur_env1 : p.E;
-    const unsigned grid = (unsigned)cdiv(a.env_end - a.env_base, b->env_group);
-    const int shape = b->env_tpb * 8 + b->env_apt;                 // (threads per block, ants per thread)
-    if (shape == 512 * 8 + 2) launch_step(b, ants::k_env<UPDATE, MOVE, 2, 512>, grid, 512u, (size_t)b->env_smem, p, a);
-    else if (shape == 512 * 8 + 1) launch_step(b, ants::k_env<UPDATE, MOVE, 1, 512>, grid, 512u, (size_t)b->env_smem, p, a);
-    else if (shape == 1024 * 8 + 1) launch_step(b, ants::k_env<UPDATE, MOVE, 1, 1024>, grid, 1024u, (size_t)b->env_smem, p, a);
-    else if (shape == 256 * 8 + 4) launch_step(b, ants::k_env<UPDATE, MOVE, 4, 256>, grid, 256u, (size_t)b->env_smem, p, a);
-    else launch_step(b, ants::k_env<UPDATE, MOVE, 1, 256>, grid, 256u, (size_t)b->env_smem, p, a);
+    const AntsBatch::Group whole = {b->stream, nullptr, 0, p.E};
+    const AntsBatch::Group *gs = b->grouped ? b->groups.data() : &whole;
+    const int n = b->grouped ? (int)b->groups.size() : 1;
+    const size_t smem = (size_t)b->env_smem;
+    a.group = b->env_group; a.cap = b->env_cap;
+    for (int k = 0; k < n; ++k) {
+        a.env_base = gs[k].env0; a.env_end = gs[k].env1;
+        const unsigned grid = (unsigned)cdiv(a.env_end - a.env_base, b->env_group);
+        {
+            LaunchScope ls(b, fam);
+            if (b->env_cap == 1024) launch_step(b, gs[k].s, ants::k_env<UPDATE, MOVE, 2, 512>, grid, 512u, smem, p, a);
+            else if (b->env_cap == 512) launch_step(b, gs[k].s, ants::k_env<UPDATE, MOVE, 1, 512>, grid, 512u, smem, p, a);
+            else launch_step(b, gs[k].s, ants::k_env<UPDATE, MOVE, 1, 256>, grid, 256u, smem, p, a);
+        }
+        TRY(check_launch(what));
+    }
+    return ANTS_OK;
+}
+
+// Lazy evaporation: no pass over the field, values are evaluated at read time from their write timestamps.  An update
+// advances the two counters the deposits are stamped with; before either wraps, one pass folds the plain values (8-byte
+// records keep 15 bits of the deposit step: expired deposits are cleared every 16384 updates, before an age of
+// tab_len <= 16384 could alias; the step counter itself keeps running).
+int advance_lazy_counters(AntsBatch *b) {
+    const Params &p = b->p;
+    const bool unbox = p.rec8 ? ((b->lazy_abs & 0x3FFFu) == 0x3FFFu) : (b->lazy_abs >= ants::kBoxMask - 2u);
+    if (b->lazy_now >= p.ts_mask - 1u || unbox) {
+        WholeBatchPass wb(b);
+        LaunchScope ls(b, F_EVAP);
+        ants::k_lazy_fold<<<148 * 16, 256, 0, b->stream>>>(p, b->lazy_now, b->lazy_abs, unbox ? 1 : 0);
+        b->lazy_now = 0;
+        if (unbox && !p.rec8) b->lazy_abs = 0;
+        TRY(check_launch("k_lazy_fold"));
+    }
+    b->lazy_now += 1;
+    b->lazy_abs += 1;
+    return ANTS_OK;
 }
 
 // host bookkeeping at the start of a step: generation folds, the step's occupancy generation, the move's arguments
@@ -476,30 +513,15 @@ void env_args_move(AntsBatch *b, const int8_t *d_rot, const int8_t *d_ph, ants::
     a->occ_gen = next_occ_gen(b);
     a->all_stamp = b->prev_synced ? 0 : 1;
     a->act_on = b->act_bool ? 1.0 : 256.0;
-    a->group = b->env_group; a->cap = b->env_apt * b->env_tpb;
 }
-// ... of an update: timestep, the lazy field's counters (a fold of plain values / expired deposits before they wrap)
+// ... of an update: timestep, the lazy field's counters
 int env_args_update(AntsBatch *b, const double *d_noise, ants::EnvArgs *a) {
-    Params &p = b->p;
     a->step_id = (uint32_t)b->timestep;
     b->timestep += 1;                                               // environment.py:45
-    if (p.P > 0 && p.lazy) {
-        const bool unbox = p.rec8 ? ((b->lazy_abs & 0x3FFFu) == 0x3FFFu) : (b->lazy_abs >= ants::kBoxMask - 2u);
-        if (b->lazy_now >= p.ts_mask - 1u || unbox) {
-            WholeBatchPass wb(b);
-            LaunchScope ls(b, F_EVAP);
-            ants::k_lazy_fold<<<148 * 16, 256, 0, b->stream>>>(p, b->lazy_now, b->lazy_abs, unbox ? 1 : 0);
-            b->lazy_now = 0;
-            if (unbox && !p.rec8) b->lazy_abs = 0;
-            TRY(check_launch("k_lazy_fold"));
-        }
-        b->lazy_now += 1;
-        b->lazy_abs += 1;
-    }
+    if (b->p.P > 0 && b->p.lazy) TRY(advance_lazy_counters(b));
     a->noise = d_noise;
     a->use_flag = b->wall_flags_valid;
     a->now = b->lazy_now; a->now_abs = b->lazy_abs;
-    a->group = b->env_group; a->cap = b->env_apt * b->env_tpb;
     return ANTS_OK;
 }
 
@@ -508,6 +530,7 @@ int finish_update(AntsBatch *b) {
     b->wall_flags_valid = 0;
     b->stats.active_tiles = 0;
     if (b->needs_sweep) {          // Anthill (order 1000) after an import: whatever the generator put into the disc (Q10)
+        WholeBatchPass wb(b);
         LaunchScope ls(b, F_ABSORB);
         ants::k_absorb_sweep<<<p.E, 256, 0, b->stream>>>(p);
         b->needs_sweep = 0;
@@ -523,11 +546,7 @@ int do_step_fused(AntsBatch *b, const int8_t *d_rot, const int8_t *d_ph, float *
     if (!b->move_done) {
         ants::EnvArgs a = {};
         env_args_move(b, d_rot, d_ph, &a);
-        {
-            LaunchScope ls(b, F_ENV_MOVE);
-            launch_env<false, true>(b, a);
-        }
-        TRY(check_launch("k_env<move>"));
+        TRY((launch_env<false, true>(b, a)));
     }
     b->move_done = 0;
     b->prev_synced = 0;
@@ -541,11 +560,7 @@ int do_step_fused(AntsBatch *b, const int8_t *d_rot, const int8_t *d_ph, float *
 int do_update_fused(AntsBatch *b, const double *d_noise) {
     ants::EnvArgs a = {};
     TRY(env_args_update(b, d_noise, &a));
-    {
-        LaunchScope ls(b, F_ENV_UPDATE);
-        launch_env<true, false>(b, a);
-    }
-    TRY(check_launch("k_env<update>"));
+    TRY((launch_env<true, false>(b, a)));
     return finish_update(b);
 }
 
@@ -557,11 +572,7 @@ int do_update_move_fused(AntsBatch *b, const int8_t *d_rot, const int8_t *d_ph) 
     TRY(env_args_update(b, nullptr, &a));
     b->prev_synced = 1;
     env_args_move(b, d_rot, d_ph, &a);
-    {
-        LaunchScope ls(b, F_ENV_FUSED);
-        launch_env<true, true>(b, a);
-    }
-    TRY(check_launch("k_env<update, move>"));
+    TRY((launch_env<true, true>(b, a)));
     b->wall_flags_valid = 0;
     b->stats.active_tiles = 0;
     b->stats.updates++;
@@ -586,69 +597,6 @@ int ensure_groups(AntsBatch *b, int want) {
         b->groups.push_back(gr);
     }
     return ANTS_OK;
-}
-
-template <typename F>
-int for_each_group(AntsBatch *b, F launch) {
-    int rc = ANTS_OK;
-    for (auto &g : b->groups) {
-        b->cur_stream = g.s; b->cur_env0 = g.env0; b->cur_env1 = g.env1;
-        rc = launch();
-        if (rc != ANTS_OK) break;
-    }
-    b->cur_stream = nullptr;
-    return rc;
-}
-
-// T x [step; update] with every kernel launched once per group of environments on the group's stream.  Host bookkeeping
-// (generation counters, lazy-field counters, timestep) advances once per step for the whole batch; the rare whole-batch
-// passes join the groups (WholeBatchPass).  Same results as the plain loop: groups share no state.
-int rollout_grouped(AntsBatch *b, const int8_t *d_rot_tape, const int8_t *d_ph_tape, int32_t n_steps, float *d_obs,
-                    float *d_as, double *d_reward) {
-    const int64_t EN = b->p.EN;
-    if (d_ph_tape && b->p.P != 2) return fail(ANTS_E_ARG, "pheromone actions need exactly two pheromones (ants.py:92-96)");
-    b->grouped = 1;
-    fork_groups(b);
-    int rc = ANTS_OK;
-    for (int t = 0; t < n_steps && rc == ANTS_OK; ++t) {
-        const int8_t *r = d_rot_tape ? d_rot_tape + (int64_t)t * EN : nullptr;
-        const int8_t *h = d_ph_tape ? d_ph_tape + (int64_t)t * EN : nullptr;
-        if (!b->move_done) {                                   // (only the first step: later moves ride on the updates)
-            ants::EnvArgs a = {};
-            env_args_move(b, r, h, &a);
-            rc = for_each_group(b, [&] { launch_env<false, true>(b, a); return check_launch("k_env<move>"); });
-            if (rc != ANTS_OK) break;
-            b->stats.kernel_launches += (int64_t)b->groups.size();
-        }
-        b->move_done = 0;
-        b->prev_synced = 0;
-        b->wall_flags_valid = 1;
-        const uint32_t og = next_obs_gen(b);
-        rc = for_each_group(b, [&] { return launch_perceive_range(b, og, d_obs, d_as, nullptr, d_reward, 1); });
-        if (rc != ANTS_OK) break;
-        b->rw_alias = 0;
-        b->stats.steps++;
-        ants::EnvArgs a = {};
-        rc = env_args_update(b, nullptr, &a);
-        if (rc != ANTS_OK) break;
-        if (t + 1 < n_steps) {
-            b->prev_synced = 1;
-            env_args_move(b, d_rot_tape ? r + EN : nullptr, d_ph_tape ? h + EN : nullptr, &a);
-            rc = for_each_group(b, [&] { launch_env<true, true>(b, a); return check_launch("k_env<update, move>"); });
-            b->move_done = 1;
-        } else {
-            rc = for_each_group(b, [&] { launch_env<true, false>(b, a); return check_launch("k_env<update>"); });
-            b->prev_synced = 1;
-        }
-        b->wall_flags_valid = 0;
-        b->stats.active_tiles = 0;
-        b->stats.updates++;
-        b->stats.kernel_launches += (int64_t)b->groups.size();     // (the perception launches count themselves)
-    }
-    join_groups(b);
-    b->grouped = 0;
-    b->cur_stream = nullptr;
-    return rc;
 }
 
 int do_observe(AntsBatch *b, float *d_obs, float *d_as, float *d_state, double *d_reward) {
@@ -679,13 +627,13 @@ int do_step(AntsBatch *b, const int8_t *d_rot, const int8_t *d_ph, float *d_obs,
     int blocks = (int)cdiv(p.EN, 256);
     {
         LaunchScope ls(b, F_MOVE);
-        launch_step(b, ants::k_step_move, (unsigned)blocks, 256u, (size_t)0, p, d_rot, d_ph, phase << 16, occ,
+        launch_step(b, b->stream, ants::k_step_move, (unsigned)blocks, 256u, (size_t)0, p, d_rot, d_ph, phase << 16, occ,
                     b->prev_synced ? 0 : 1, b->act_bool ? 1.0 : 256.0, b->commit_par);
     }
     TRY(check_launch("k_step_move"));
     {
         LaunchScope ls(b, F_FOOD);
-        launch_step(b, ants::k_food_commit, 64u, 128u, (size_t)0, p, phase << 16, b->absorb_par, b->commit_par);
+        launch_step(b, b->stream, ants::k_food_commit, 64u, 128u, (size_t)0, p, phase << 16, b->absorb_par, b->commit_par);
         b->commit_par ^= 1;
     }
     TRY(check_launch("k_food_commit"));
@@ -709,7 +657,7 @@ int do_update(AntsBatch *b, const double *d_noise) {
     //    nothing the objects in between read.
     {
         LaunchScope ls(b, F_COLLIDE);
-        launch_step(b, ants::k_collide, (unsigned)blocks, 256u, (size_t)0, p, d_noise, step_id, phase << 16,
+        launch_step(b, b->stream, ants::k_collide, (unsigned)blocks, 256u, (size_t)0, p, d_noise, step_id, phase << 16,
                     p.R > 0 ? 0 : 1, b->wall_flags_valid, b->absorb_par);
         b->absorb_par ^= 1;
         b->wall_flags_valid = 0;
@@ -719,30 +667,19 @@ int do_update(AntsBatch *b, const double *d_noise) {
     if (p.R > 0) {
         {
             LaunchScope ls(b, F_ROCKS);
-            launch_step(b, ants::k_rocks_pushed, (unsigned)cdiv((int64_t)p.E * p.R, 8), 256u, (size_t)0, p);
+            launch_step(b, b->stream, ants::k_rocks_pushed, (unsigned)cdiv((int64_t)p.E * p.R, 8), 256u, (size_t)0, p);
         }
         TRY(check_launch("k_rocks_pushed"));
         {
             LaunchScope ls(b, F_ROCKS);
-            launch_step(b, ants::k_rocks_push_ants, (unsigned)blocks, 256u, (size_t)0, p, phase << 16);
+            launch_step(b, b->stream, ants::k_rocks_push_ants, (unsigned)blocks, 256u, (size_t)0, p, phase << 16);
         }
         TRY(check_launch("k_rocks_push_ants"));
     }
     // 1b + 4. wall zeroing of the field (walls.py:30) and Pheromone.update (order 0)
     if (p.P > 0) {
         if (p.lazy) {
-            // no pass over the field: values are evaluated at read time from their write timestamps
-            // (8-byte records keep 15 bits of the deposit step: expired deposits are cleared every 16384 updates,
-            //  before an age of tab_len <= 16384 could alias; the step counter itself keeps running)
-            const bool unbox = p.rec8 ? ((b->lazy_abs & 0x3FFFu) == 0x3FFFu) : (b->lazy_abs >= ants::kBoxMask - 2u);
-            if (b->lazy_now >= p.ts_mask - 1u || unbox) {     // fold before a counter wraps
-                LaunchScope ls(b, F_EVAP);
-                ants::k_lazy_fold<<<148 * 16, 256, 0, b->stream>>>(p, b->lazy_now, b->lazy_abs, unbox ? 1 : 0);
-                b->lazy_now = 0;
-                if (unbox && !p.rec8) b->lazy_abs = 0;
-            }
-            b->lazy_now += 1;
-            b->lazy_abs += 1;
+            TRY(advance_lazy_counters(b));
             b->stats.active_tiles = 0;
         } else if (b->cfg.diffuse_factor != 0.0) {
             int nbx = (int)cdiv(p.W, ants::kStX), nby = (int)cdiv(p.H, ants::kStY);
@@ -772,7 +709,8 @@ int do_update(AntsBatch *b, const double *d_noise) {
         // 6. Ants.update (order 999): deposit
         {
             LaunchScope ls(b, F_DEPOSIT);
-            launch_step(b, ants::k_deposit_commit, (unsigned)blocks, 256u, (size_t)0, p, phase << 16, b->lazy_now, b->lazy_abs);
+            launch_step(b, b->stream, ants::k_deposit_commit, (unsigned)blocks, 256u, (size_t)0, p, phase << 16,
+                        b->lazy_now, b->lazy_abs);
         }
         TRY(check_launch("k_deposit_commit"));
     }
@@ -1022,12 +960,7 @@ int ants_create(const AntsConfig *cfg, AntsBatch **out) {
         b->fused = ((p.lazy || p.P == 0) && cfg->diffuse_factor == 0.0 && p.N <= 1024 && p.plane < 0xFFFFFFF0ll &&
                     !getenv("ANTS_NO_FUSED")) ? 1 : 0;
         b->env_group = g;
-        // block shape: one ant per thread up to 512 ants per block; a 1024-ant block as 512 threads x 2 ants (measured
-        // on the cfg4 shard: 0.090 ms against 0.111 for 256 x 4 and 0.098 for 1024 x 1; ANTS_ENV_TPB selects those)
-        b->env_tpb = cap <= 256 ? 256 : 512;
-        if (cap == 1024)
-            if (const char *x = getenv("ANTS_ENV_TPB")) { const int t = atoi(x); if (t == 256 || t == 1024) b->env_tpb = t; }
-        b->env_apt = cap / b->env_tpb;
+        b->env_cap = cap;
         // The block-per-environment kernel is heavy (256 threads x 64 registers, 33 KB of shared memory): launched as a
         // programmatic dependent it sits on the SMs waiting for the perception kernel and takes registers and shared
         // memory from it (measured: rollouts 0.37-0.61 ms per step against 0.36 for separate launches), so the pair
@@ -1170,8 +1103,6 @@ int ants_create(const AntsConfig *cfg, AntsBatch **out) {
         // add/subtract wraps them unless the map is smaller than that
         double reach = p.radius * cfg->delta * 1.5 + fabs(cfg->fwd_delta) + 2.0;
         b->perceive_slow_wrap = (p.W <= reach || p.H <= reach) ? 1 : 0;
-        // fewer resident blocks leave more of the 228 KB SM array to the L1 cache, which serves the record re-reads
-        if (const char *x = getenv("ANTS_PERCEIVE_PAD_SMEM")) b->perceive_smem += atoi(x);
     }
     {   // straight-line perception code for the generator's default channel list (with / without rocks)
         const int std6[6] = {ANTS_CH_ANTS, ANTS_CH_PHERO, ANTS_CH_PHERO, ANTS_CH_ANTHILL, ANTS_CH_WALLS, ANTS_CH_FOOD};
@@ -1739,37 +1670,35 @@ int ants_rollout(AntsBatch *b, const int8_t *d_rot_tape, const int8_t *d_ph_tape
     const int64_t EN = b->p.EN;
     if (n_steps <= 0) return ANTS_OK;
     if (!d_obs || !d_agent_state) return fail(ANTS_E_ARG, "ants_rollout: obs and agent_state buffers are required");
-    {   // groups of environments on their own streams: large batches on the block-per-env kernels (ANTS_ROLLOUT_GROUPS
-        // overrides: 1 = off)
-        int want = (b->fused && b->perceive_rows && EN >= 131072) ? 4 : 1;
-        if (const char *x = getenv("ANTS_ROLLOUT_GROUPS")) want = atoi(x);
-        if (want > 1 && b->fused && b->perceive_rows && !b->profiling) {
-            if (b->needs_sweep) {                              // first update after an import: the plain path sweeps the hill
-                const int8_t *r0 = d_rot_tape, *h0 = d_ph_tape;
-                TRY(do_step(b, r0, h0, d_obs, d_agent_state, d_reward, nullptr));
-                TRY(do_update(b, nullptr));
-                if (n_steps == 1) return ANTS_OK;
-                d_rot_tape = d_rot_tape ? d_rot_tape + EN : nullptr;
-                d_ph_tape = d_ph_tape ? d_ph_tape + EN : nullptr;
-                n_steps -= 1;
-            }
-            TRY(ensure_groups(b, want));
-            if (b->groups.size() > 1) return rollout_grouped(b, d_rot_tape, d_ph_tape, n_steps, d_obs, d_agent_state, d_reward);
-        }
+    if (d_ph_tape && b->p.P != 2)
+        return fail(ANTS_E_ARG, "pheromone actions need exactly two pheromones (ants.py:92-96), have %d", b->p.P);
+    // Groups of environments on streams of their own for large batches on the block-per-env kernels
+    // (ANTS_ROLLOUT_GROUPS overrides: 1 = off).  The step kernels launch once per group; host bookkeeping (generation
+    // counters, lazy-field counters, timestep) advances once per step for the whole batch, and the rare whole-batch
+    // passes (folds, the anthill sweep after an import) join the groups first.  Groups share no state: the results are
+    // those of the plain loop.
+    int want = (b->fused && b->perceive_rows && EN >= 131072) ? 4 : 1;
+    if (const char *x = getenv("ANTS_ROLLOUT_GROUPS")) want = atoi(x);
+    if (want > 1 && b->fused && b->perceive_rows && !b->profiling) {
+        TRY(ensure_groups(b, want));
+        b->grouped = b->groups.size() > 1 ? 1 : 0;
+        if (b->grouped) fork_groups(b);
     }
-    for (int t = 0; t < n_steps; ++t) {
+    int rc = ANTS_OK;
+    for (int t = 0; t < n_steps && rc == ANTS_OK; ++t) {
         const int8_t *r = d_rot_tape ? d_rot_tape + (int64_t)t * EN : nullptr;
         const int8_t *h = d_ph_tape ? d_ph_tape + (int64_t)t * EN : nullptr;
-        TRY(do_step(b, r, h, d_obs, d_agent_state, d_reward, nullptr));
-        if (b->fused && t + 1 < n_steps && !b->needs_sweep) {
-            // update_t and the move of step_{t+1} in one launch; do_step(t + 1) then only perceives
-            if (h && b->p.P != 2) return fail(ANTS_E_ARG, "pheromone actions need exactly two pheromones");
-            TRY(do_update_move_fused(b, d_rot_tape ? r + EN : nullptr, d_ph_tape ? h + EN : nullptr));
-        } else {
-            TRY(do_update(b, nullptr));
-        }
+        rc = do_step(b, r, h, d_obs, d_agent_state, d_reward, nullptr);
+        if (rc != ANTS_OK) break;
+        // update_t and the move of step_{t+1} in one launch; do_step(t + 1) then only perceives
+        if (b->fused && t + 1 < n_steps && !b->needs_sweep)
+            rc = do_update_move_fused(b, d_rot_tape ? r + EN : nullptr, d_ph_tape ? h + EN : nullptr);
+        else
+            rc = do_update(b, nullptr);
     }
-    return ANTS_OK;
+    if (b->grouped) join_groups(b);
+    b->grouped = 0;
+    return rc;
 }
 
 int ants_sample_actions(AntsBatch *b, uint64_t seed, int32_t n_rotations, int32_t n_pheromones, int8_t *d_rot,

@@ -5,15 +5,15 @@
 // last-writer scatters of the reference (quirk Q1: ants.py:116, pheromone.py:39), the ordered sum of the ants' pushes
 // on a rock (circle_obstacles.py:38-40) -- and resolve the scatters through a global `owner` array (atomicMax per ant,
 // re-read by a follow-up kernel: two random DRAM sectors per ant and scatter).  Here a block owns G consecutive
-// environments (G * N <= CAP ants, CAP in {256, 512, 1024}: 256 or 512 threads with one ant each, or 512 threads with two
-// for the 1024-ant block -- measured 0.090 ms on the cfg4 shard against 0.111 for 256 x 4 and 0.098 for 1024 x 1), so those
-// phase boundaries are block barriers, the owner of a cell is found in a shared-memory hash table
-// (cell -> highest ant index, atomicCAS / atomicMax on shared memory) and the rock pushes are summed from positions
-// staged in shared memory.  Per iteration of `update(); step()` the ants' state is read and written once, and the
-// record of the cell an ant stands on is loaded once for the pheromone deposit (update) AND the mandible rule of the
-// next step (RL_api.py:178-185: after an update prev_ants == ants, so it is the same cell and the same winner).
+// environments (G * N <= CAP ants, CAP in {256, 512, 1024}: 256 or 512 threads with one ant each, or 512 threads with
+// two for the 1024-ant block), so those phase boundaries are block barriers, the owner of a cell is found in a
+// shared-memory hash table (cell -> highest ant index, atomicCAS / atomicMax on shared memory) and the rock pushes are
+// summed from positions staged in shared memory.  Per iteration of `update(); step()` the ants' state is read and
+// written once, and the record of the cell an ant stands on is loaded once for the pheromone deposit (update) AND the
+// mandible rule of the next step (RL_api.py:178-185: after an update prev_ants == ants, so it is the same cell and the
+// same winner).
 //
-//   k_env<UPDATE, MOVE, APT>:
+//   k_env<UPDATE, MOVE, APT, TPB>:
 //     UPDATE: Environment.update() (environment.py:42-47) for lazy-evaporation handles: Anthill absorb of the cells
 //             queued by the previous move (anthill.py:41-46), Walls.update on ants (walls.py:24-28),
 //             CircleObstacles.update (circle_obstacles.py:32-58), the ant part of Ants.update (ants.py:123-130) and
@@ -23,6 +23,12 @@
 //   <1,0> = ants_update, <0,1> = first half of ants_step, <1,1> = update_k ; step_{k+1} inside ants_rollout.
 // Used when the field is lazy (or there are no pheromones), N <= 1024 and the keys fit 32 bits; everything else keeps
 // the flat kernels (ANTS_NO_FUSED forces them, for A/B tests).
+//
+// Measured on the cfg4 shard (512 envs x 1024 ants, 8-byte records, one B200) and left out of the code again:
+//   * the 1024-ant block as 256 threads x 4 ants or 1024 x 1: 0.111 and 0.098 ms against 0.090 for 512 x 2;
+//   * update+move: the move ahead of the mandible rule, again where the holding changes: 0.111 against 0.098 ms;
+//   * the move's occupancy stamp as a store without a load, the wall bit read by the update: 0.117 against 0.101 ms;
+//   * the per-ant helpers (wrap, sincos, food load, deposit) called instead of inlined: 0.103 against 0.098 ms.
 #pragma once
 
 namespace ants {
@@ -81,25 +87,11 @@ __device__ __forceinline__ void prefetch_l2(const void *ptr) { asm volatile("pre
 // Heavy or rare pieces of the per-ant work are kept out of line: the kernel body is unrolled over the ants of a thread,
 // and inlining them four times made it 12 000 instructions (ncu: 2.5 stall cycles per instruction waiting for the
 // instruction cache).
-#ifndef ANTS_ENV_HOT_INLINE
-#define ANTS_ENV_HOT_INLINE 1      // the helpers every ant runs (wrap, sincos, food load, deposit): inline (1) or called (0)
-#endif
-#ifndef ANTS_ENV_SPECULATE
-#define ANTS_ENV_SPECULATE 0       // update+move: move before the mandible rule, again for the ants whose holding changes
-                                   // (measured slower: 0.111 against 0.098 ms on the cfg4 shard)
-#endif
-#if ANTS_ENV_HOT_INLINE
-#define ANTS_ENV_HOT __forceinline__
-#else
-#define ANTS_ENV_HOT __noinline__
-#endif
-__device__ ANTS_ENV_HOT double env_wrap(double v, double n) { return pymod_near(v, n); }
-__device__ ANTS_ENV_HOT void env_sincos(double t, double *s, double *c) { sincos(t, s, c); }
 __device__ __noinline__ double env_noise(const Params &p, int e, uint32_t step_id, int ant) {
     return philox_uniform(p.rng_seed, (uint32_t)(p.env_id_base + e), step_id, (uint32_t)ant);
 }
 // the owner of a cell adds its activations and clamps (ants.py:98-100, pheromone.py:36-41)
-__device__ ANTS_ENV_HOT void env_deposit(const Params &p, uint8_t *rec, int64_t i, uint32_t now, uint32_t now_abs, double av0, double av1) {
+__device__ __forceinline__ void env_deposit(const Params &p, uint8_t *rec, int64_t i, uint32_t now, uint32_t now_abs, double av0, double av1) {
     for (int q = 0; q < p.P; ++q) {
         const double av = q == 0 ? av0 : (q == 1 ? av1 : p.act[(int64_t)q * p.EN + i]);   // (the first two were loaded with the ant state)
         if (av == 0.0) continue;
@@ -113,7 +105,6 @@ __device__ __noinline__ double env_food_commit(const Params &p, uint8_t *fr, dou
     st_food(p, fr, v);
     return ld_food(p, fr);
 }
-__device__ ANTS_ENV_HOT double env_ld_food(const Params &p, const uint8_t *r) { return ld_food(p, r); }
 
 // the rock-grid entries follow a rock that moved (clear the old box, set the new one); a whole warp calls this
 __device__ __noinline__ void env_move_rock_grid(const Params &p, int e, int r, double cx, double cy, double nx, double ny, double rad, int lane) {
@@ -159,21 +150,13 @@ __device__ __noinline__ void env_push_by_rocks(const Params &p, int e, unsigned 
             sx += vx * fac; sy += vy * fac;
         }
     }
-    *x = env_wrap(*x + sx, (double)p.W);                               // translate_ants -> warp_xy
-    *y = env_wrap(*y + sy, (double)p.H);
+    *x = pymod_near(*x + sx, (double)p.W);                             // translate_ants -> warp_xy
+    *y = pymod_near(*y + sy, (double)p.H);
 }
 
-#ifndef ANTS_ENV_WALLFLAG
-#define ANTS_ENV_WALLFLAG 1        // 1: the move reads the record of the new cell (prefetched) and leaves its wall bit in
-                                   //    wall_hit[] for the coming update; 0: the move only stores the occupancy stamp and the
-                                   //    update reads the wall bit with the record it needs anyway -- one random sector less
-                                   //    per ant, but a dependent DRAM load at the head of the kernel: 0.117 against 0.101 ms
-#endif
-#ifndef ANTS_ENV_MINBLOCKS
-#define ANTS_ENV_MINBLOCKS 4       // resident blocks per SM the register budget allows (4 x 256 threads x 64 registers)
-#endif
-template <bool UPDATE, bool MOVE, int APT, int TPB = kEnvThreads>
-__global__ void __launch_bounds__(TPB, (ANTS_ENV_MINBLOCKS * kEnvThreads) / TPB)
+constexpr int kEnvMinBlocks = 4;   // resident 256-thread blocks per SM at 64 registers
+template <bool UPDATE, bool MOVE, int APT, int TPB>
+__global__ void __launch_bounds__(TPB, (kEnvMinBlocks * kEnvThreads) / TPB)
 k_env(const __grid_constant__ Params p, const EnvArgs a) {
     pdl_begin();
     constexpr int CAP = APT * TPB;
@@ -212,8 +195,7 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
     // together, with the index of an idle slot clamped to the block's last ant: the kernel lives on memory-level
     // parallelism (two random DRAM sectors per ant: the cell it deposits on and the cell it moves to).
     double th[APT];
-    int newcell[APT];              // MOVE: the cell the ant moves to ...
-    int newxy[APT];                // ... and its coordinates (x << 16 | y)
+    int newcell[APT];              // MOVE: the cell the ant moves to
     int cell[APT];                 // UPDATE: the cell the ant ends the update in; MOVE alone: its prev cell
     int el[APT];                   // environment within the block
     int lac[APT];                  // the ant's slot in the block (clamped)
@@ -224,7 +206,7 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
         valid[k] = la < n_loc;
         lac[k] = valid[k] ? la : (n_loc - 1);
         el[k] = a.group == 1 ? 0 : lac[k] / p.N;
-        th[k] = 0.0; cell[k] = 0; newcell[k] = 0; newxy[k] = 0;
+        th[k] = 0.0; cell[k] = 0; newcell[k] = 0;
     }
     // record of cell c of the block's env g: (g * plane + c) fits 32 bits (the hash keys rely on the same bound)
     uint8_t *const cells0 = p.cells + (((int64_t)env0 * p.plane) << p.rec_shift);
@@ -241,7 +223,7 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
         for (int k = 0; k < APT; ++k) {
             const int64_t i = i0 + lac[k];
             x[k] = p.x[i]; y[k] = p.y[i]; th[k] = p.theta[i];
-            in_wall[k] = (ANTS_ENV_WALLFLAG && a.use_flag) ? p.wall_hit[i] != 0 : false;
+            in_wall[k] = a.use_flag ? p.wall_hit[i] != 0 : false;
             // what the later phases read, requested now (no registers held): the activations of the depositing owners,
             // the ant state of the move
             if (p.P > 0) { prefetch_l2(p.act + i); if (p.P > 1) prefetch_l2(p.act + p.EN + i); }
@@ -273,10 +255,9 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
         if (tid < n_env) p.absorb_count[env0 + tid] = 0u;
         // ---- Walls.update on ants (walls.py:24-28) + which rocks does an ant push (circle_obstacles.py:35-37)
         const int Gc = ((p.N + 31) / 32 + 31) / 32 * 32;               // ants per touch chunk (<= 32 chunks)
-        // Walls.update (walls.py:24-25): the wall bit of the cell the ant stands on.  This is the ONE random DRAM sector of
-        // the ant per iteration: unless a wall or a rock moves it, it is also the cell it deposits on and the cell whose
-        // food the mandible rule reads (the move of the previous step only stored the occupancy stamp there).
-        if (!(ANTS_ENV_WALLFLAG && a.use_flag)) {
+        // Walls.update (walls.py:24-25): the wall bit of the cell the ant stands on, left in wall_hit[] by the move of
+        // the previous step; without such a move (an update after an import or another update) read from the record
+        if (!a.use_flag) {
 #pragma unroll
             for (int k = 0; k < APT; ++k)
                 in_wall[k] = ld_wall(p, rec_of(el[k], cidx(p, cell_of(x[k], W), cell_of(y[k], H))));
@@ -357,14 +338,8 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
         }
         // ---- prev snapshot and reward_state decay (ants.py:124,130), ownership of the deposit cell (pheromone.py:39, Q1)
         uint8_t rs[APT];
-        double hold0[APT];
-        int8_t rot0[APT];
 #pragma unroll
-        for (int k = 0; k < APT; ++k) {
-            const int64_t i = i0 + lac[k];
-            rs[k] = p.reward_state[i];
-            if (MOVE) { hold0[k] = p.holding[i]; rot0[k] = a.rot != nullptr ? a.rot[i] : (int8_t)0; }
-        }
+        for (int k = 0; k < APT; ++k) rs[k] = p.reward_state[i0 + lac[k]];
 #pragma unroll
         for (int k = 0; k < APT; ++k) {
             if (!valid[k]) continue;
@@ -378,24 +353,6 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
             if (p.P > 0 || MOVE) {
                 prefetch_l2(rec_of(el[k], cell[k]));                   // consumed after the barrier
                 env_hash_max(hkeys, hvals, HMASK, (uint32_t)(el[k] * p.plane + cell[k]) + 1u, (uint32_t)ant + 1u);
-            }
-            if (MOVE && ANTS_ENV_SPECULATE) {
-                // The move of the coming step (ants.py:62-80), ahead of the mandible rule: heading and rotation do not
-                // depend on the food, the speed only through the holding of an ant that picks up or drops in this very
-                // step -- those few are moved again below.  This takes the record of the NEW cell (a second random
-                // DRAM sector) out of the dependency chain behind the record of the current one.
-                double t = th[k];
-                if (a.rot != nullptr) t = env_wrap(t + (double)rot0[k] * p.max_rot_speed, 6.283185307179586);    // ants.py:62-67
-                double fwd = (1.0 * p.max_speed) * (1.0 - hold0[k] * p.csr);            // RL_api.py:194
-                if (fwd < 0.0) fwd *= p.bsr;                                            // RL_api.py:195
-                double sn, cs;
-                env_sincos(t, &sn, &cs);
-                const double x1 = env_wrap(x[k] + cs * fwd, Wd);                        // ants.py:69-80
-                const double y1 = env_wrap(y[k] + sn * fwd, Hd);
-                p.x[i] = x1; p.y[i] = y1; p.theta[i] = t;
-                const int nx = cell_of(x1, W), ny = cell_of(y1, H);
-                newcell[k] = cidx(p, nx, ny); newxy[k] = (nx << 16) | ny;
-                if (ANTS_ENV_WALLFLAG) prefetch_l2(rec_of(el[k], newcell[k]));
             }
         }
         __syncthreads();
@@ -417,7 +374,7 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
 #pragma unroll
         for (int k = 0; k < APT; ++k) {
             cell[k] = cidx(p, cell_of(px[k], W), cell_of(py[k], H));
-            fd[k] = env_ld_food(p, rec_of(el[k], cell[k]));
+            fd[k] = ld_food(p, rec_of(el[k], cell[k]));
         }
 #pragma unroll
         for (int k = 0; k < APT; ++k) {
@@ -441,7 +398,7 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
         for (int k = 0; k < APT; ++k) {
             const int64_t i = i0 + lac[k];
             hold[k] = p.holding[i]; mand[k] = p.mandibles[i];
-            rot[k] = (!(UPDATE && ANTS_ENV_SPECULATE) && a.rot != nullptr) ? a.rot[i] : (int8_t)0;
+            rot[k] = a.rot != nullptr ? a.rot[i] : (int8_t)0;
             phv[k] = a.ph != nullptr ? a.ph[i] : (int8_t)0;
         }
     }
@@ -454,7 +411,7 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
     }
     if (UPDATE && MOVE) {
 #pragma unroll
-        for (int k = 0; k < APT; ++k) fd[k] = env_ld_food(p, rec_of(el[k], cell[k]));   // prev cell == this cell after an update
+        for (int k = 0; k < APT; ++k) fd[k] = ld_food(p, rec_of(el[k], cell[k]));   // prev cell == this cell after an update
     }
 #pragma unroll
     for (int k = 0; k < APT; ++k) {
@@ -482,23 +439,17 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
             // (after an update the prev cell IS the current cell: its hill bit decides whether dropped food is queued)
             flags[k] = (own ? 1 : 0) | (delta != 0.0 ? 2 : 0) | ((UPDATE && hill) ? 4 : 0);
             fd[k] = fd[k] + delta;                                                      // what the owner will write (ants.py:116)
-            constexpr bool kSpec = UPDATE && (ANTS_ENV_SPECULATE != 0);
-            if (!kSpec || h != hold[k]) {
-                // MOVE alone: the move itself.  After an update it already ran with the old holding (above): only an
-                // ant whose holding just changed moves again, with the speed that goes with it
-                double t = kSpec ? p.theta[i] : th[k];
-                if (!kSpec && a.rot != nullptr) t = env_wrap(t + (double)rot[k] * p.max_rot_speed, 6.283185307179586);   // ants.py:62-67
-                double fwd = (1.0 * p.max_speed) * (1.0 - h * p.csr);                   // RL_api.py:194
-                if (fwd < 0.0) fwd *= p.bsr;                                            // RL_api.py:195
-                double sn, cs;
-                env_sincos(t, &sn, &cs);
-                const double x = env_wrap(x0 + cs * fwd, Wd);                           // ants.py:69-80
-                const double y = env_wrap(y0 + sn * fwd, Hd);
-                p.x[i] = x; p.y[i] = y; p.theta[i] = t;
-                const int nx = cell_of(x, W), ny = cell_of(y, H);
-                newcell[k] = cidx(p, nx, ny); newxy[k] = (nx << 16) | ny;
-                if (ANTS_ENV_WALLFLAG) prefetch_l2(rec_of(el[k], newcell[k]));
-            }
+            double t = th[k];
+            if (a.rot != nullptr) t = pymod_near(t + (double)rot[k] * p.max_rot_speed, 6.283185307179586);   // ants.py:62-67
+            double fwd = (1.0 * p.max_speed) * (1.0 - h * p.csr);                       // RL_api.py:194
+            if (fwd < 0.0) fwd *= p.bsr;                                                // RL_api.py:195
+            double sn, cs;
+            sincos(t, &sn, &cs);
+            const double x = pymod_near(x0 + cs * fwd, Wd);                             // ants.py:69-80
+            const double y = pymod_near(y0 + sn * fwd, Hd);
+            p.x[i] = x; p.y[i] = y; p.theta[i] = t;
+            newcell[k] = cidx(p, cell_of(x, W), cell_of(y, H));
+            prefetch_l2(rec_of(el[k], newcell[k]));
         }
     }
     if (!MOVE) return;
@@ -533,33 +484,22 @@ k_env(const __grid_constant__ Params p, const EnvArgs a) {
             p.act[p.EN + i] = (v != 0 && v != 1) ? a.act_on : 0.0;
         }
     }
-    // Occupancy stamp of the new cell (RL_api.py:136-142) and its wall bit for the coming update.  (ANTS_ENV_WALLFLAG = 0:
-    // the stamp as a store without a load -- the byte it shares with the anthill bit of the compact records is rebuilt from
-    // the disc test on integers, the same test k_hill_mark wrote the bit with -- and the wall bit read by the update.)
+    // Occupancy stamp of the new cell (RL_api.py:136-142) and its wall bit for the coming update
     // (the loads of all the thread's ants first, then the stores: a load behind a store is not moved up by the compiler)
     uint32_t meta[APT];            // compact records: the 16 bits [hill | occ stamp][wall | explored stamp]; else the wall bit
-    if (ANTS_ENV_WALLFLAG) {
 #pragma unroll
-        for (int k = 0; k < APT; ++k) {
-            const uint8_t *orec = rec_of(el[k], newcell[k]);
-            meta[k] = (p.rec8 || p.rec16) ? (uint32_t)*reinterpret_cast<const uint16_t *>(orec + (p.rec8 ? 6 : 12))
-                                          : (ld_wall(p, orec) ? 0x8000u : 0u);
-        }
+    for (int k = 0; k < APT; ++k) {
+        const uint8_t *orec = rec_of(el[k], newcell[k]);
+        meta[k] = (p.rec8 || p.rec16) ? (uint32_t)*reinterpret_cast<const uint16_t *>(orec + (p.rec8 ? 6 : 12))
+                                      : (ld_wall(p, orec) ? 0x8000u : 0u);
     }
 #pragma unroll
     for (int k = 0; k < APT; ++k) {
         if (!valid[k]) continue;
         uint8_t *orec = rec_of(el[k], newcell[k]);
-        if (ANTS_ENV_WALLFLAG) {
-            p.wall_hit[i0 + lac[k]] = (uint8_t)(meta[k] >> 15);        // for Walls.update of the coming update
-            if (p.rec8 || p.rec16) orec[p.rec8 ? 6 : 12] = (uint8_t)((meta[k] & 0x80u) | (a.occ_gen & 0x7Fu));
-            else st_occ(p, orec, a.occ_gen);
-        } else if (p.rec8 || p.rec16) {
-            const bool hill = in_hill(p.hill + 4 * (env0 + el[k]), newxy[k] >> 16, newxy[k] & 0xFFFF);
-            orec[p.rec8 ? 6 : 12] = (uint8_t)((hill ? 0x80u : 0u) | (a.occ_gen & 0x7Fu));
-        } else {
-            st_occ(p, orec, a.occ_gen);
-        }
+        p.wall_hit[i0 + lac[k]] = (uint8_t)(meta[k] >> 15);            // for Walls.update of the coming update
+        if (p.rec8 || p.rec16) orec[p.rec8 ? 6 : 12] = (uint8_t)((meta[k] & 0x80u) | (a.occ_gen & 0x7Fu));
+        else st_occ(p, orec, a.occ_gen);
     }
 }
 

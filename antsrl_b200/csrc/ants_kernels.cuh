@@ -1158,11 +1158,7 @@ __global__ void __launch_bounds__(256) k_evaporate_tiles(Params p, const uint32_
 // instruction, scripts/microbench/tma_probe.cu -- so the box starts two columns left of the tile: 66 x 68.)
 // tile shape (measured on 1024 envs x 256^2, 2 pheromones, ms per update): 32x32 0.488, 16x64 0.474, 8x128 0.468,
 // 64x32 0.407, 128x32 0.360, 64x64 0.354 (= 0.96 of the measured HBM copy peak)
-#ifndef ANTS_ST_X
-#define ANTS_ST_X 64
-#define ANTS_ST_Y 64
-#endif
-constexpr int kStX = ANTS_ST_X, kStY = ANTS_ST_Y, kStPadY = 2;
+constexpr int kStX = 64, kStY = 64, kStPadY = 2;
 // Arithmetic: a warp owns 32 columns and a few consecutive output rows; a thread slides down its column
 // keeping per input row the three clipped values (left, centre, right), their sum and the sum of the two sides, so an
 // output costs 3 shared-memory loads and ~10 f64 operations instead of 9 and 27:

@@ -27,10 +27,8 @@
 
 namespace ants {
 
-#ifndef ANTS_ROWS_THREADS
-#define ANTS_ROWS_THREADS 32
-#endif
-constexpr int kRowsThreads = ANTS_ROWS_THREADS;
+constexpr int kRowsThreads = 32;
+constexpr int kRowsOcc = 20;         // resident one-warp blocks per SM: 20 warps at 96 registers
 constexpr int kRowsGroup = 4;
 constexpr int kRowsTiles = 1;        // staging tiles per warp
 
@@ -86,10 +84,6 @@ __device__ __noinline__ float rock_channel(const Params &p, int e, unsigned long
     return 0.f;
 }
 
-template <int LAYOUT, int REC, int S>      // REC: 0 = f64 records, 1 = compact 16-byte, 2 = compact 8-byte
-#ifndef ANTS_ROWS_OCC
-#define ANTS_ROWS_OCC (5 * 128 / ANTS_ROWS_THREADS)   // resident warps per SM / warps per block: 20 warps at 96 registers
-#endif
 // Measured on the cfg4 shard (512 envs x 1024 ants, 8-byte records, one B200) and left out of the code again:
 //   * all 32 * S rows of a warp handed to the lanes without idle lanes (two staging tiles): 0.279 ms against 0.241;
 //   * the record loads of chunk g + 1 issued before chunk g is decoded (two register sets): 0.278 - 0.338 ms;
@@ -106,7 +100,8 @@ template <int LAYOUT, int REC, int S>      // REC: 0 = f64 records, 1 = compact 
 //   * 2 or 3 ants per thread in phases A / C (a warp serving 64 or 96 ants, the round trips of phase A paid once for all
 //     of them; prep record cut to 64 bytes with the first rock's disc re-read from global memory): 0.247 and 0.282 ms
 //     against 0.189 for the same code with one ant per thread (profiles/r2_bench/perceive_variants_apt.txt).
-__global__ void __launch_bounds__(kRowsThreads, ANTS_ROWS_OCC)
+template <int LAYOUT, int REC, int S>      // REC: 0 = f64 records, 1 = compact 16-byte, 2 = compact 8-byte
+__global__ void __launch_bounds__(kRowsThreads, kRowsOcc)
 k_perceive_rows(const __grid_constant__ Params p, float *__restrict__ obs, float *__restrict__ agent_state, float *__restrict__ state_out,
                 double *__restrict__ reward_out, uint32_t obs_gen, uint32_t occ_gen, int is_step, int rw_alias,
                 uint32_t now, uint32_t now_abs, int64_t ant0, int64_t ant_end) {

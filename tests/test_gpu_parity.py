@@ -229,25 +229,29 @@ def test_lazy_timestamp_fold():
 @pytest.mark.parametrize("record,n_rocks", [("compact8", 0), ("compact8", 4), ("compact", 0), ("f64", 4)])
 def test_rollout_equals_step_update_loop(record, n_rocks, groups, monkeypatch):
     """ants_rollout (device-resident action tapes, C loop; optionally the batch as groups of environments on streams of
-    their own) == the same steps issued one by one."""
+    their own) == the same steps issued one by one.  6 envs of 100 ants are 3 blocks of the block-per-env kernel (2 envs
+    each), so three groups get one block each; the rollout starts with the anthill sweep of the import pending."""
     import torch
     monkeypatch.setenv("ANTS_ROLLOUT_GROUPS", str(groups))
     from antsrl_b200 import BatchedAnts
-    scen = [make_scenario(seed=800 + e, w=48, h=48, n_ants=40, n_rocks=n_rocks, steps=12, n_walls=6) for e in range(3)]
+    T, E = 12, 6
+    scen = [make_scenario(seed=800 + e, w=48, h=48, n_ants=100, n_rocks=n_rocks, steps=T, n_walls=6) for e in range(E)]
     cfg = scen[0][0]
-    rot = torch.from_numpy(np.stack([[s[2]["rot"][t] for s in scen] for t in range(12)])).cuda().contiguous()
-    ph = torch.from_numpy(np.stack([[s[2]["ph"][t] for s in scen] for t in range(12)])).cuda().contiguous()
+    rot = torch.from_numpy(np.stack([[s[2]["rot"][t] for s in scen] for t in range(T)])).cuda().contiguous()
+    ph = torch.from_numpy(np.stack([[s[2]["ph"][t] for s in scen] for t in range(T)])).cuda().contiguous()
     outs = []
     for mode in ("loop", "rollout"):
-        b = BatchedAnts(cfg, 3, evap_mode="lazy", record=record, rng_seed=3)
+        b = BatchedAnts(cfg, E, evap_mode="lazy", record=record, rng_seed=3)
         b.import_state(stack_init(cfg, [i for _, i, _ in scen]))
         b.observe()
         if mode == "loop":
-            for t in range(12):
+            for t in range(T):
                 obs, ast, rew, _ = b.step(rot[t], ph[t])
                 b.update(None)
         else:
+            launches = b.stats()["kernel_launches"]
             obs, ast, rew = b.rollout(rot, ph)
+            assert b.stats()["kernel_launches"] - launches >= 2 * groups * T      # every step kernel once per group
         st = b.export_state()
         outs.append((obs.cpu().numpy().copy(), rew.cpu().numpy().copy(), st))
         b.close()
@@ -618,22 +622,11 @@ def test_partial_import_keeps_scalars():
     b.close()
 
 
-@pytest.mark.parametrize("tpb", [256, 1024])
-def test_block_shapes_of_the_env_kernel(tpb, monkeypatch):
-    """The 1024-ant block of k_env as 256 threads x 4 ants and as 1024 x 1 (ANTS_ENV_TPB; the default 512 x 2 runs in
-    every other 513..1024-ant test): a rollout and a step / update loop against the oracle."""
-    monkeypatch.setenv("ANTS_ENV_TPB", str(tpb))
-    test_rollout_matches_oracle("compact8", 5, 1000, 2, 1, monkeypatch)
-    kw = dict(seed=1800, w=72, h=64, n_ants=700, n_rocks=4, steps=12, n_walls=5, n_food=12)
-    rep = run_parity(_variants(kw, 2), evap_mode="lazy", record="compact8")
-    assert rep["state_checks"] == 12
-
-
 @pytest.mark.parametrize("groups", [1, 4], ids=["one_stream", "four_groups"])
 @pytest.mark.parametrize("record,n_rocks,n_ants,n_envs", [("compact8", 6, 300, 3), ("compact8", 0, 50, 7), ("compact", 4, 520, 2),
                                                           ("f64", 3, 1024, 2), ("compact8", 2, 1100, 2)])
 def test_rollout_matches_oracle(record, n_rocks, n_ants, n_envs, groups, monkeypatch):
-    """ants_rollout (update_k and the move of step_{k+1} in ONE launch of the block-per-environment kernel; 1, 2 or 4
+    """ants_rollout (update_k and the move of step_{k+1} in ONE launch of the block-per-environment kernel; 1 or 2
     ants per thread, several envs per block for small N; 1100 ants per env falls back to the flat kernels) against the
     oracle: last observation / reward and the full final state after 30 steps, Philox noise, crowded hill (shared
     cells: the last-writer scatters) and food near it."""
@@ -718,14 +711,17 @@ def test_windowed_import_resets_some_environments(record, n_rocks):
 
 
 def test_grouped_rollout_crosses_generation_folds(monkeypatch):
-    """150 steps of ants_rollout with the batch split into groups on their own streams: the 7-bit generation counters of
-    the compact records fold on the way (whole-batch passes that must join the groups first and fork them again)."""
+    """260 steps of ants_rollout with the batch split into groups on their own streams: the 7-bit generation counters of
+    the compact records fold twice on the way and the lazy field's update counter once (whole-batch passes that must
+    join the groups first and fork them again).  12 envs of 48 ants are 3 blocks of the block-per-env kernel (5 envs
+    each, the last one partial), one per group."""
     import torch
     from antsrl_b200 import BatchedAnts
     from oracle.antsrl_oracle import OracleEnv, philox_uniform
     from parity_util import compare_state
-    monkeypatch.setenv("ANTS_ROLLOUT_GROUPS", "2")
-    T, E, N = 150, 4, 48
+    G = 3
+    monkeypatch.setenv("ANTS_ROLLOUT_GROUPS", str(G))
+    T, E, N = 260, 12, 48
     scen = [make_scenario(seed=1700 + e, w=64, h=56, n_ants=N, n_rocks=3, steps=T, n_walls=5, n_food=8) for e in range(E)]
     cfg = scen[0][0]
     oracles = [OracleEnv(c, i) for c, i, _ in scen]
@@ -736,8 +732,10 @@ def test_grouped_rollout_crosses_generation_folds(monkeypatch):
         o.observation()
     rot = torch.from_numpy(np.stack([[s[2]["rot"][t] for s in scen] for t in range(T)])).cuda().contiguous()
     ph = torch.from_numpy(np.stack([[s[2]["ph"][t] for s in scen] for t in range(T)])).cuda().contiguous()
+    launches = b.stats()["kernel_launches"]
     obs, ast, rew = b.rollout(rot[:100], ph[:100])           # two calls: the second one starts with move_done cleared
     obs, ast, rew = b.rollout(rot[100:], ph[100:])
+    launches = b.stats()["kernel_launches"] - launches
     refs = []
     for e, o in enumerate(oracles):
         for t in range(T):
@@ -746,7 +744,7 @@ def test_grouped_rollout_crosses_generation_folds(monkeypatch):
         refs.append(r)
     _cmp_outputs((obs, ast, rew), refs, "last step of the grouped rollout")
     compare_state(b.export_state(), oracles, "after the grouped rollout", cfg)
-    assert b.stats()["kernel_launches"] > 2 * T
+    assert launches >= 2 * G * T                               # every step kernel once per group
     b.close()
 
 

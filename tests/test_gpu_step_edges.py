@@ -818,14 +818,6 @@ def test_step_update_loop_fused(name, rec):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("tpb", ("256", "1024"))
-def test_fused_1024_ant_block_shapes(tpb, monkeypatch):
-    """The 1024-ant block as 256 threads x 4 ants and 1024 x 1."""
-    monkeypatch.setenv("ANTS_ENV_TPB", tpb)
-    run_loop(*worlds_of("n1000"), record="compact8")
-
-
-@pytest.mark.gpu
 @pytest.mark.parametrize("path", ("fused", "flat"))
 @pytest.mark.parametrize("mode", range(5))
 def test_mandible_rule_modes(mode, path, monkeypatch):
