@@ -1218,6 +1218,24 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     Params &p = b->p;
     if (env0 < 0 || n_envs < 1 || (int64_t)env0 + n_envs > p.E)
         return fail(ANTS_E_ARG, "env window [%d, %d) outside the batch of %d envs", env0, env0 + n_envs, p.E);
+    // the per-ant and rock arrays (kilobytes per env) are checked here, before anything is uploaded: the handle stays as
+    // it was.  A NaN or infinite value has no counterpart the kernels could follow (NaN positions index no cell, and a
+    // NaN activation would deposit a saturated trail where the reference's convolution spreads NaN).
+    const size_t an_all = (size_t)n_envs * p.N;
+    const struct { const char *name; const double *v; size_t n, per_env; } finite[] = {
+        {"x", s->x, an_all, (size_t)p.N}, {"y", s->y, an_all, (size_t)p.N}, {"theta", s->theta, an_all, (size_t)p.N},
+        {"prev_x", s->prev_x, an_all, (size_t)p.N}, {"prev_y", s->prev_y, an_all, (size_t)p.N},
+        {"prev_theta", s->prev_theta, an_all, (size_t)p.N}, {"holding", s->holding, an_all, (size_t)p.N},
+        {"activation", s->activation, an_all * p.P, (size_t)p.N * p.P},
+        {"rock_centers", s->rock_centers, (size_t)n_envs * p.R * 2, (size_t)p.R * 2},
+        {"rock_radii", s->rock_radii, (size_t)n_envs * p.R, (size_t)p.R},
+        {"rock_weights", s->rock_weights, (size_t)n_envs * p.R, (size_t)p.R}};
+    for (const auto &f : finite)
+        if (f.v)
+            for (size_t i = 0; i < f.n; ++i)
+                if (!std::isfinite(f.v[i]))
+                    return fail(ANTS_E_ARG, "env %d: %s[%zu] is %g; imported values must be finite", env0 + (int)(i / f.per_env),
+                                f.name, i % f.per_env, f.v[i]);
     if (p.diffuse && s->activation) {                  // a plane value's sign bit is the wall flag: no negative deposits
         const size_t n = (size_t)n_envs * p.N * p.P;
         for (size_t i = 0; i < n; ++i)
@@ -1258,19 +1276,22 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     // map fields: dense host array -> device scratch -> pack kernel into the cell records
     const size_t ncell = (size_t)n_envs * p.W * p.H;
     Scratch scratch;
-    size_t scratch_flag_off = 0;                                           // one word after the data: k_plane_walls's flag
+    uint32_t *d_bad = nullptr;                                             // one word after the data: the kBad* flags
     if (s->phero || s->food || s->walls || s->explored) {
         size_t need = ncell * 8 * ((s->phero && p.P > 1) ? p.P : 1);
-        scratch_flag_off = need;
+        const size_t flag_off = need;
         need += sizeof(uint32_t);
         cudaError_t me = cudaMalloc(&scratch.ptr, need);
         if (me != cudaSuccess) return fail(ANTS_E_ALLOC, "import scratch of %zu bytes: %s", need, cudaGetErrorString(me));
+        d_bad = (uint32_t *)((char *)scratch.ptr + flag_off);
+        CK(cudaMemsetAsync(d_bad, 0, sizeof(uint32_t), st));
     }
     void *const d_tmp = scratch.ptr;
     if (s->phero && p.P > 0) {
         CK(cudaMemcpyAsync(d_tmp, s->phero, ncell * 8 * p.P, cudaMemcpyHostToDevice, st));
         for (int k = 0; k < p.P; ++k)
-            ants::k_pack_f64<<<148 * 8, 256, 0, st>>>(p, (const double *)d_tmp, p.P, k, 8 * k, k, b->lazy_now, b->lazy_abs, env0, n_envs);
+            ants::k_pack_f64<<<148 * 8, 256, 0, st>>>(p, (const double *)d_tmp, p.P, k, 8 * k, k, b->lazy_now, b->lazy_abs,
+                                                      env0, n_envs, d_bad);
         TRY(check_launch("k_pack_f64"));
         if (p.tile_active) {
             ants::k_tiles_from_phero<<<148 * 4, 256, 0, st>>>(p, env0, n_envs);
@@ -1279,7 +1300,8 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     }
     if (s->food) {
         CK(cudaMemcpyAsync(d_tmp, s->food, ncell * 8, cudaMemcpyHostToDevice, st));
-        ants::k_pack_f64<<<148 * 8, 256, 0, st>>>(p, (const double *)d_tmp, 1, 0, p.food_off, -1, 0u, 0u, env0, n_envs);
+        ants::k_pack_f64<<<148 * 8, 256, 0, st>>>(p, (const double *)d_tmp, 1, 0, p.food_off, -1, 0u, 0u, env0, n_envs,
+                                                  d_bad);
         TRY(check_launch("k_pack_f64"));
         b->needs_sweep = 1;
     }
@@ -1288,14 +1310,12 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
         ants::k_pack_u8<<<148 * 8, 256, 0, st>>>(p, (const uint8_t *)d_tmp, 0, env0, n_envs);      // Walls.__init__: astype(bool)
         TRY(check_launch("k_pack_u8"));
     }
-    uint32_t bad_phero = 0;
     if (p.diffuse && (s->walls || s->phero)) {         // the planes carry the wall bit in their sign
-        uint32_t *d_bad = s->phero ? (uint32_t *)((char *)d_tmp + scratch_flag_off) : nullptr;
-        if (d_bad) CK(cudaMemsetAsync(d_bad, 0, sizeof(uint32_t), st));
-        ants::k_plane_walls<<<148 * 8, 256, 0, st>>>(p, env0, n_envs, d_bad);
+        ants::k_plane_walls<<<148 * 8, 256, 0, st>>>(p, env0, n_envs, s->phero ? d_bad : nullptr);
         TRY(check_launch("k_plane_walls"));
-        if (d_bad) CK(cudaMemcpyAsync(&bad_phero, d_bad, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     }
+    uint32_t bad = 0;
+    if (d_bad) CK(cudaMemcpyAsync(&bad, d_bad, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     if (s->explored) {
         CK(cudaMemcpyAsync(d_tmp, s->explored, ncell, cudaMemcpyHostToDevice, st));
         ants::k_pack_u8<<<148 * 8, 256, 0, st>>>(p, (const uint8_t *)d_tmp, 1, env0, n_envs);
@@ -1344,7 +1364,12 @@ int ants_import_env_state(AntsBatch *b, int32_t env0, int32_t n_envs, const Ants
     if (s->rw_alias >= 0) b->rw_alias = s->rw_alias ? 1 : 0;
     if (s->act_bool >= 0) b->act_bool = s->act_bool ? 1 : 0;
     CK(cudaStreamSynchronize(st));   // host temporaries above must outlive the copies
-    if (bad_phero)
+    if (bad & ants::kBadNonFinite)
+        return fail(ANTS_E_ARG, "an imported pheromone or food value is NaN or infinite (import the window again)");
+    if (bad & ants::kBadAboveMax)
+        return fail(ANTS_E_ARG, "an imported pheromone value is above max_val %g; lazy fields hold values <= max_val "
+                    "(import the window again)", p.phero_max_val);
+    if (bad & ants::kBadNegative)
         return fail(ANTS_E_ARG, "an imported pheromone value is negative or NaN; with diffusion values must be >= 0 "
                     "(import the window again)");
     return ANTS_OK;
@@ -1633,6 +1658,9 @@ int ants_activate_all_pheromones(AntsBatch *b, const double *act, int32_t is_boo
     for (int64_t i = 0; i < p.EN; ++i)
         for (int k = 0; k < p.P; ++k) {
             double v = act[i * p.P + k];
+            if (!is_bool && !std::isfinite(v))         // (bool activations map NaN to 1, as numpy's astype(bool))
+                return fail(ANTS_E_ARG, "env %d, ant %d: activation %g; activations must be finite", (int)(i / p.N),
+                            (int)(i % p.N), v);
             if (p.diffuse && !is_bool && !(v >= 0.0))  // a plane value's sign bit is the wall flag: no negative deposits
                 return fail(ANTS_E_ARG, "env %d, ant %d: activation %g; with diffusion an activation must be >= 0",
                             (int)(i / p.N), (int)(i % p.N), v);

@@ -1223,9 +1223,18 @@ k_diffuse_tma(Params p, const __grid_constant__ CUtensorMap tmap, int src_z0, in
         }
     }
 }
-// after an import: the sign bit of every plane value = the wall bit of its cell record.  `bad` (non-null when the
-// planes were just imported, so they still hold the caller's values): set to 1 if one of them is negative or NaN --
-// the sign bit is the wall flag, so such a value cannot be represented (ants_import_env_state rejects the import)
+// Bits of an import's flag word (`bad`, the scratch word after the imported data), which ants_import_env_state
+// returns as ANTS_E_ARG once the window's import has run:
+//   kBadNonFinite  a pheromone or food value is NaN or +-inf (k_pack_f64): a deposit's fmin would turn a NaN into a
+//                  saturated deposit, a NaN record reads as the boxed deposit of update 0, and the reference's
+//                  convolution spreads the NaN to the neighbours -- not emulated
+//   kBadAboveMax   lazy mode with max_val: a pheromone value above max_val (k_pack_f64).  The reference clamps it inside
+//                  the next update, after evaporation (pheromone.py:41 after :44-45); a plain lazy record cannot, and
+//                  the reference's own updates never leave such a value (each one clamps the whole plane)
+//   kBadNegative   diffusion: a negative or NaN plane value (k_plane_walls); its sign bit would be read as the wall flag
+constexpr uint32_t kBadNonFinite = 1u, kBadAboveMax = 2u, kBadNegative = 4u;
+// after an import: the sign bit of every plane value = the wall bit of its cell record.  `bad` is non-null when the
+// planes were just imported, so they still hold the caller's values.
 __global__ void k_plane_walls(Params p, int env0, int n_env, uint32_t *bad) {
     const int64_t n = (int64_t)n_env * p.W * p.H;
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
@@ -1238,7 +1247,7 @@ __global__ void k_plane_walls(Params p, int env0, int n_env, uint32_t *bad) {
         for (int k = 0; k < p.P; ++k) {
             double *pv = plane_at(p, (int)e, k, x, y);
             const double v = *pv, a = fabs(v);
-            if (bad != nullptr && !(v >= 0.0)) *bad = 1u;
+            if (bad != nullptr && !(v >= 0.0)) atomicOr(bad, kBadNegative);
             *pv = wall ? -a : a;
         }
     }
@@ -1311,8 +1320,9 @@ __global__ void __launch_bounds__(256) k_absorb_sweep(Params p) {
 
 // ------------------------------------------------------------------------------------------------ import / export helpers
 // dense host-layout arrays <-> record fields.  `dense` is [E][planes_per_env][W][H]; field = plane `k` of them.
+// `bad`: the import's flag word (kBad* above).
 __global__ void k_pack_f64(Params p, const double *__restrict__ dense, int planes_per_env, int k, int byte_off,
-                           int phero_k, uint32_t now, uint32_t now_abs, int env0, int n_env) {
+                           int phero_k, uint32_t now, uint32_t now_abs, int env0, int n_env, uint32_t *bad) {
     const int64_t n = (int64_t)n_env * p.W * p.H;
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
         int64_t ex = j / p.H;
@@ -1320,12 +1330,13 @@ __global__ void k_pack_f64(Params p, const double *__restrict__ dense, int plane
         int64_t e = ex / p.W;                                                  // position in the imported window
         int x = (int)(ex - e * p.W);
         double v = dense[((e * planes_per_env + k) * p.W + x) * p.H + y];
+        if (!isfinite(v)) atomicOr(bad, kBadNonFinite);
+        else if (phero_k >= 0 && p.lazy && p.has_max_val && v > p.phero_max_val) atomicOr(bad, kBadAboveMax);
         e += env0;
         uint8_t *r = rec_at(p, (int)e, cidx(p, x, y));
         if (phero_k >= 0 && p.diffuse) {
             *plane_at(p, (int)e, phero_k, x, y) = v;                           // (k_plane_walls sets the sign afterwards)
         } else if (phero_k >= 0) {
-            if (p.lazy && p.has_max_val) v = fmin(v, p.phero_max_val);         // pheromone.py:41 (applied at import)
             phero_store(p, r, phero_k, v, now, now_abs);
         } else {
             st_food(p, r, v);
